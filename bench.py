@@ -5,12 +5,13 @@ Workload at every N (weak scaling): BASELINE config 2 -- FNO2dObserver(12,12,32)
 4 Fourier layers, 128x128 synthetic vorticity-like fields, batch 64 PER GPU, fp32.  One step = forward,
 relative-L2 loss (run_pde_observers.py:138,188-193), backward, (N>1: one NCCL gradient all-reduce), Adam.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
-Prints ONE JSON line (rank 0).  `value` = device-timed throughput with inputs resident in HBM; `e2e` =
+Prints ONE JSON line (rank 0).  `value` = device-timed throughput of K steps with inputs resident in HBM; `e2e` =
 the same through the public module API with pinned HOST inputs (H2D + loss D2H inside the timed region).
-`--impl reference` times the reference's CPU algorithm (oracle port; /root/reference does not travel to
-the GPU box) on the host cores with all threads, on a bounded sample of the same workload.
+`--impl reference` times the reference's CPU algorithm (the oracle port, or the unmodified reference where
+B2NO_REFERENCE_ROOT names a checkout of it) on the host cores with all threads, on a bounded sample of the same workload.
+`--dump-outputs DIR` writes what the last timed step computed as .npy files (dump_outputs()).
 """
 import argparse
 import json
@@ -128,7 +129,7 @@ class ClockSampler:
 # ---------------------------------------------------------------------------------------------
 def cpu_reference_run(steps, warmup, sample_batch):
     """Times fwd + rel-L2 + bwd + Adam of FNO2dObserver on the CPU with every host thread.
-    Uses the unmodified reference when /root/reference exists (kind 'reference'), else the oracle port."""
+    Uses the unmodified reference when B2NO_REFERENCE_ROOT names a checkout of it (kind 'reference'), else the oracle port."""
     from oracle import ref_loader, restated as rs
     torch.set_num_threads(os.cpu_count() or 1)
     torch.manual_seed(0)
@@ -475,6 +476,25 @@ def other_configs(dev, rank, world, timed, args):
     return out
 
 
+def dump_outputs(out_dir, loss, model):
+    """What the timed training step computed in its last step: the loss it returned, and the parameters (after the Adam
+    update) and gradients it left in the model, as float32 .npy files (complex tensors as (..., 2) real views), ~5 MB in
+    all.  The batch and the initial weights are seeded and the timed steps start from those weights, so two builds run with
+    the same arguments compare file by file.  Some gradient reductions are not bitwise deterministic and training on one
+    batch amplifies their rounding, so --steps 1 gives the tightest comparison."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss}
+    for name, p in model.named_parameters():
+        arrays[f"param.{name}"] = p
+        if p.grad is not None:
+            arrays[f"grad.{name}"] = p.grad
+    for name, t in arrays.items():
+        t = t.detach()
+        t = torch.view_as_real(t) if t.is_complex() else t
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 # ---------------------------------------------------------------------------------------------
 def run_b200(args):
     import pde_policylearning_b200 as P
@@ -547,6 +567,10 @@ def run_b200(args):
 
     # resident inputs: the graph's static buffers already hold this rank's batch -> no copies in the timed region
     res_in = (graphed.static_in[0], graphed.static_tgt) if graphed is not None else (p_dev, t_dev)
+    # The warm-up steps below train the model too; their updates are undone before the timed region, so the K timed steps
+    # start from the seeded initial weights in every run (--dump-outputs with --steps 1 is one step on identical inputs)
+    opt_state = (opt.flat_param, opt.exp_avg, opt.exp_avg_sq, opt.step_counter)
+    init_state = [t.clone() for t in opt_state]
     # clock / power pre-warm (untimed, not part of W): a GPU that sat idle through the host-side set-up measured its first
     # 20 steps 9 % slow (2.61 vs 2.38 ms, profiles/r02_l) -- run the step ~0.3 s worth of times before the W warm-up steps
     # A FIXED number of steps: the step contains the gradient all-reduce at N > 1, so every rank must run the same count
@@ -556,27 +580,33 @@ def run_b200(args):
     torch.cuda.synchronize()
     for _ in range(args.warmup):
         step(*res_in)
+    for dst, src in zip(opt_state, init_state):
+        dst.copy_(src)
     l0 = ops.launch_count()
-    # The K-step region (barrier + synchronize on both sides, device-timed, max over ranks) is measured three times back to
-    # back and the MEDIAN is reported: the region is ~45 ms long, and at N = 8 one host-side hiccup on any of the eight ranks
-    # (every step ends in an all-reduce) was seen to double a single measurement (5.13 vs 2.30 ms per step).  All three
-    # figures go into the JSON line (config.timed_region_ms).  The cyclic GC is off for the duration.
+    # The K-step region: barrier + synchronize on both sides, device-timed, max over ranks.  The cyclic GC is off for the
+    # duration.  The loss of every step is kept (a list assignment on the host) so that --dump-outputs sees the last one.
     import gc
     gc.collect()
     gc.disable()
+    last = [None]
+
+    def timed_step():
+        last[0] = step(*res_in)
+
     with ClockSampler(local_rank) as clk:
-        reps_ms = [timed(lambda: step(*res_in), args.steps) for _ in range(3)]
+        ms = timed(timed_step, args.steps)
     gc.enable()
-    ms = sorted(reps_ms)[1]
-    launches = (ops.launch_count() - l0) // (3 * args.steps)
+    launches = (ops.launch_count() - l0) // args.steps
     clocks = clk.summary()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last[0], model)
     ms_per_step = ms / args.steps
     value = BATCH * world / (ms_per_step * 1e-3)
 
     if args.quick:
         if rank == 0:
             emit(json.dumps({"metric": METRIC, "value": round(value, 2), "ms_per_step": round(ms_per_step, 4), "n_gpus": world,
-                             "clocks": clocks, "quick": True, "timed_region_ms": [round(v, 3) for v in reps_ms]}))
+                             "clocks": clocks, "quick": True, "timed_region_ms": round(ms, 3)}))
         if world > 1:
             dist.barrier()
             if graphed is not None:
@@ -650,9 +680,8 @@ def run_b200(args):
         cfg = config_dict(world)
         cfg["cuda_graph"] = graphed is not None
         cfg["prewarm_steps"] = 120          # untimed, before the W warm-up steps (fixed count: same on every rank)
-        cfg["timed_region_ms"] = [round(v, 3) for v in reps_ms]
-        cfg["timing"] = (f"median of 3 back-to-back repetitions of the {args.steps}-step region, each bracketed by barrier + "
-                         "synchronize, CUDA events, max over ranks")
+        cfg["timed_region_ms"] = round(ms, 3)
+        cfg["timing"] = f"one {args.steps}-step region bracketed by barrier + synchronize, CUDA events, max over ranks"
         cfg["optimizer"] = "fused flat Adam (lr 1e-3, weight_decay 1e-4), inside the timed step"
         cfg["grad_allreduce"] = ("none (1 GPU)" if world == 1 else
                                  ("per-bucket NCCL all-reduce launched from gradient hooks during backward (B2NO_OVERLAP_AR=1)"
@@ -766,7 +795,13 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="run the training step eagerly instead of as one CUDA graph")
     ap.add_argument("--no-other", action="store_true", help="skip the cfg3 / cfg4 / cfg5 measurements (other_configs)")
     ap.add_argument("--only", default=None, choices=["cfg3", "cfg4", "cfg5"], help="measure one of the other configs alone")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss, parameters and gradients of the last timed step to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.only):
+        ap.error("--dump-outputs applies to the b200 training step (not --impl reference or --only)")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)

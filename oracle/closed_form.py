@@ -10,8 +10,8 @@ convolutions compute:
 All three are  rfftn -> keep low modes -> per-mode channel mixing -> irfftn.  Here the same map is
 written as explicit mode-restricted DFT matrices in complex128, together with the hand-derived
 backward (dx, dW, dbias).  It is the *specification* the CUDA kernels are tested against; it is
-pinned against the reference itself (tests/test_oracle_vs_reference.py, run where /root/reference
-exists) and against the committed fixtures in tests/golden/ (generated from the reference by
+pinned against the reference itself (tests/test_oracle_vs_reference.py, run where B2NO_REFERENCE_ROOT
+names a checkout of it) and against the committed fixtures in tests/golden/ (generated from the reference by
 tests/golden/make_golden.py).
 
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline leg may import this module; the

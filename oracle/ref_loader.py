@@ -4,17 +4,17 @@ Only ``tests/``, ``tests/golden/make_golden.py``, ``__graft_entry__.smoke()`` an
 ``cpu_baseline`` / ``--impl reference`` legs of ``bench.py`` may import this file.
 The product package (``pde_policylearning_b200``) never does.
 
-The reference (``/root/reference``) is pure Python/PyTorch but its ``neuralop`` half
+The reference (a checkout of it, named by ``B2NO_REFERENCE_ROOT``) is pure Python/PyTorch but its ``neuralop`` half
 imports ``tensorly`` / ``tltorch`` / ``torch_harmonics`` which are not installed and
 cannot be installed (no network).  SURVEY.md Appendix A lists the exact third-party
 surface the dense path touches; this file registers in-memory stand-ins for those
 names (parameter *storage* only -- every arithmetic op stays ``torch.fft`` /
 ``torch.einsum``) and then imports the reference files from where they lie.  Nothing
-is copied out of ``/root/reference``.
+is copied out of the checkout.
 
-``/root/reference`` exists only in the build container, not on the GPU box, so
-``available()`` must be checked first; everything that has to travel is turned into
-fixtures under ``tests/golden/`` by ``tests/golden/make_golden.py``.
+The reference is not part of this repository, so ``available()`` must be checked first;
+what the tests need from it is turned into fixtures under ``tests/golden/`` by
+``tests/golden/make_golden.py``.
 """
 from __future__ import annotations
 
@@ -26,11 +26,11 @@ import types
 import torch
 from torch import nn
 
-REFERENCE_ROOT = os.environ.get("B2NO_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("B2NO_REFERENCE_ROOT", "")
 
 
 def available() -> bool:
-    return os.path.isdir(os.path.join(REFERENCE_ROOT, "neuralop", "models"))
+    return bool(REFERENCE_ROOT) and os.path.isdir(os.path.join(REFERENCE_ROOT, "neuralop", "models"))
 
 
 # --------------------------------------------------------------------------------------

@@ -4,11 +4,11 @@ Functional PyTorch (torch.fft + einsum, autograd) re-expressions of the referenc
 hot path, driven by a ``state_dict`` with the reference's own key names.  They follow the reference's
 *algorithm* (full rfftn, slice corners, einsum, scatter into zeros, irfftn), i.e. what the reference's CPU
 path does -- this is what ``bench.py``'s ``cpu_baseline`` / ``--impl reference`` legs time on the GPU
-box's host cores (``kind: "port"``; /root/reference does not exist there) and what the model-level
+machine's host cores (``kind: "port"`` where no checkout of the reference is named) and what the model-level
 parity tests compare against at sizes too large for committed fixtures.
 
-Pinned against the reference itself in tests/test_oracle_vs_reference.py (runs where /root/reference
-exists) and against tests/golden/*.pt (generated from the reference by tests/golden/make_golden.py).
+Pinned against the reference itself in tests/test_oracle_vs_reference.py (runs where B2NO_REFERENCE_ROOT
+names a checkout of it) and against tests/golden/*.pt (generated from the reference by tests/golden/make_golden.py).
 
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / reference legs may import this.
 """

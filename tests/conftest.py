@@ -20,11 +20,14 @@ def pytest_configure(config):
 def golden():
     import torch
 
+    import seeded_inputs
+
     cache = {}
 
     def load(name):
         if name not in cache:
-            cache[name] = torch.load(os.path.join(GOLDEN, name + ".pt"), map_location="cpu", weights_only=False)
+            data = torch.load(os.path.join(GOLDEN, name + ".pt"), map_location="cpu", weights_only=False)
+            cache[name] = seeded_inputs.restore(name, data)
         return cache[name]
 
     return load

@@ -1,6 +1,6 @@
 """CPU: the oracle (closed form + restated models) against the committed golden vectors, which were produced
-by the UNMODIFIED reference (tests/golden/make_golden.py).  This is what pins the oracle on boxes where
-/root/reference does not exist."""
+by the UNMODIFIED reference (tests/golden/make_golden.py).  This is what pins the oracle where no
+checkout of the reference is at hand."""
 import pytest
 import torch
 
