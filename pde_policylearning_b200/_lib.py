@@ -9,7 +9,7 @@ import subprocess
 import sys
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# B2NO_LIB: load another build of the same sources (A/B measurements of compile-time switches)
+# B2NO_LIB: load another build, e.g. the parent commit's, for A/B runs in one call
 LIB_PATH = os.environ.get("B2NO_LIB") or os.path.join(_HERE, "libb2no.so")
 CSRC = os.path.join(_HERE, "csrc")
 SOURCES = ["plan.cu", "spectral.cu", "pointwise.cu", "tc_pointwise.cu", "tc_wgrad.cu", "tc_mlp.cu", "tc_head_bwd.cu", "tc_dft.cu", "tc_mix.cu", "tc_peak.cu", "pino_loss.cu", "optim.cu"]
@@ -41,13 +41,6 @@ class Epilogue(C.Structure):
 
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-Xcompiler", "-fPIC"]
 HEADERS = [os.path.join(CSRC, "common.cuh"), os.path.join(CSRC, "tc.cuh"), os.path.join(_HERE, "..", "include", "b2no.h")]
-
-
-def nvcc_command(out_path: str = LIB_PATH, defines=()):
-    """The one-shot form of the build (all sources in one nvcc call); build() compiles the same sources with the same
-    flags file by file, in parallel, and links the objects."""
-    srcs = [os.path.join(CSRC, s) for s in SOURCES]
-    return ["nvcc"] + NVCC_FLAGS + ["-shared"] + [f"-D{d}" for d in defines] + ["-o", out_path] + srcs
 
 
 def build(force: bool = False, verbose: bool = False) -> str:

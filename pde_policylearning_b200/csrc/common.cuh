@@ -19,14 +19,6 @@ extern long long g_b2no_launches;
     g_b2no_launches++;                             \
   } while (0)
 
-// debug / ablation switches are environment variables read ONCE per process (never on the launch path)
-#include <stdlib.h>
-static inline int b2no_env_int(const char* name, int dflt) {
-  const char* e = getenv(name);
-  return (e && e[0]) ? atoi(e) : dflt;
-}
-#define B2NO_ENV_ONCE(var, name, dflt) static const int var = b2no_env_int(name, dflt)
-
 static inline int b2no_ceil_div(long a, long b) { return (int)((a + b - 1) / b); }
 static inline int b2no_round_up(int a, int b) { return ((a + b - 1) / b) * b; }
 

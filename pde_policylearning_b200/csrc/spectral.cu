@@ -459,8 +459,7 @@ extern "C" int b2no_dft_forward(const b2no_plan* p, int which, const float* x, f
   if (d == 1) return run_r2c(p, which, x, spec, bc, st);
   if (d == 2) {
     // small planes (RNO 32 x 32): one warp per plane on the FMA pipe -- the 128-row tensor-core tile is four planes there
-    B2NO_ENV_ONCE(env_small, "B2NO_FWD_SMALL", 1);
-    if (env_small && n[0] <= 32 && n[1] <= 32 && n[1] % 4 == 0 && p->K[0] <= 32 && Kl <= 16 && (((uintptr_t)x) & 15) == 0 &&
+    if (n[0] <= 32 && n[1] <= 32 && n[1] % 4 == 0 && p->K[0] <= 32 && Kl <= 16 && (((uintptr_t)x) & 15) == 0 &&
         (p->g.spec_layout == 0 || p->g.spec_layout == 1))
       return launch_fwd_plane32(p, which, x, spec, (long)bc, st);
     // tensor-core path (tc_dft.cu): one kernel, no intermediate, when the plane shape fits the 128-row tile

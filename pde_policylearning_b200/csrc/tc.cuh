@@ -26,28 +26,14 @@ __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
 __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
 }
-// The wait suspends the warp in hardware for up to kMbarSuspendNs before the instruction returns false (PTX: the optional
-// suspendTimeHint of mbarrier.try_wait).  Without the hint a waiting warp came back every ~30 ns: in the persistent
-// kernels here a quarter of all issued instructions were TRYWAIT / BRA / YIELD of warps that had nothing to do, taken
-// from the issue slots of the epilogue warps sharing their scheduler.
-// Measured (B200): the hint removes the polling instructions but changes no kernel time, and a warp woken from the
-// suspended wait sees the barrier ~0.08 us later than a polling one (k_wgrad_tc hand-over stamps) -- so the default is
-// the plain polling wait; -DB2NO_MBAR_HINT_NS=20000 builds the suspended variant.
-#ifndef B2NO_MBAR_HINT_NS
-#define B2NO_MBAR_HINT_NS 0
-#endif
-constexpr uint32_t kMbarSuspendNs = B2NO_MBAR_HINT_NS;
+// A plain polling wait.  Without a suspend hint a waiting warp comes back every ~30 ns: in the persistent kernels here a
+// quarter of all issued instructions were TRYWAIT / BRA / YIELD of warps that had nothing to do, taken from the issue
+// slots of the epilogue warps sharing their scheduler.  Measured (B200): the optional suspendTimeHint of mbarrier.try_wait
+// removes those polling instructions but changes no kernel time, and a warp woken from the suspended wait sees the
+// barrier ~0.08 us later than a polling one (k_wgrad_tc hand-overs); a nanosleep back-off after a failed poll changed
+// nothing either.
 __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
   uint32_t ok;
-#if B2NO_MBAR_HINT_NS > 0
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity), "r"(kMbarSuspendNs)
-      : "memory");
-#else
   asm volatile(
       "{\n\t.reg .pred p;\n\t"
       "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
@@ -55,19 +41,10 @@ __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
       : "=r"(ok)
       : "r"(smem_u32(bar)), "r"(parity)
       : "memory");
-#endif
   return ok != 0;
 }
-// -DB2NO_MBAR_SLEEP_NS=n: back off n ns after a failed poll (fewer try_wait requests in the shared-memory pipe)
-#ifndef B2NO_MBAR_SLEEP_NS
-#define B2NO_MBAR_SLEEP_NS 0
-#endif
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  while (!mbar_try_wait(bar, parity)) {
-#if B2NO_MBAR_SLEEP_NS > 0
-    __nanosleep(B2NO_MBAR_SLEEP_NS);
-#endif
-  }
+  while (!mbar_try_wait(bar, parity)) {}
 }
 
 // explicit shared-space accesses on 32-bit addresses (a generic pointer into shared memory compiles to ST.E / LD.E on the
@@ -259,11 +236,7 @@ __device__ __forceinline__ float tf32_rna(float x) {
 // lo = x - trunc(x) is exact in fp32 (it is the low 13 mantissa bits); the tensor core then reads ITS upper 19 bits, i.e.
 // truncates it to 10 mantissa bits: hi + lo carries 21 mantissa bits, error 2^-21 relative to x.  Rounding lo first (cvt.rna,
 // an XU-pipe instruction with a long latency, one per element in every converter loop) would only gain the last half bit.
-#ifdef B2NO_LO_RNA
-__device__ __forceinline__ float tf32_lo(float x) { return tf32_rna(x - tf32_trunc(x)); }
-#else
 __device__ __forceinline__ float tf32_lo(float x) { return x - tf32_trunc(x); }
-#endif
 
 // K-major, no-swizzle ("interleaved") canonical layout for 4-byte elements: core matrix = 8 rows x 16 B.
 // Element (r, k) of an [R x K] operand lives at byte offset

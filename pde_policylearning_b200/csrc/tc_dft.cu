@@ -39,7 +39,6 @@ struct FdTc {
   long tiles, tiles_per_cta, planes;
   const float* tb; const float* mimg;
   float* spec;
-  int debug;   // ablation switches (B2NO_FD_DEBUG): 1 no converter TMEM stores, 2 no MMAs, 4 no hand-over stores, 8 no lo split
   int npass;   // 3: 3xTF32, 1: single-pass TF32 (never merged)
   int layout;  // 0: spectrum (plane, kx, ky); 1: mode-major (kx, ky, plane)
 };
@@ -65,16 +64,6 @@ __host__ __device__ inline FdLayout fd_layout(const FdTc& p) {
   return L;
 }
 
-// debug: %globaltimer stamps of CTA 0 (B2NO_FD_DEBUG & 16), read back with b2no_debug_fd_ts
-__device__ unsigned long long g_fd_ts[16];
-__device__ __forceinline__ void fd_stamp(const FdTc& p, int slot) {
-  if ((p.debug & 16) && blockIdx.x == 0) {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-    g_fd_ts[slot] = t;
-  }
-}
-
 // warp roles (16 warps; a warp may only touch TMEM lanes 32 * (warp % 4) .. + 31)
 //   0-3   converter A (even K chunks)      4-7  converter B (odd K chunks)      8-9  spectrum write-out (lanes 0-63)
 //   10    TMA producer                     11   MMA issuer                      12-15 hand-over D1 -> stage-2 B operand
@@ -98,7 +87,6 @@ k_fwd_tc(const __grid_constant__ CUtensorMap tmx, const FdTc p) {
   uint32_t* tslot = (uint32_t*)(mt_staged + 1);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int N1 = p.N1, H = p.H, R = p.R, nk = p.nk;
-  if (tid == 0) fd_stamp(p, 0);
 
   // ---- one-time setup ----
   {
@@ -125,7 +113,6 @@ k_fwd_tc(const __grid_constant__ CUtensorMap tmx, const FdTc p) {
   __syncthreads();
   tc_fence_after();
   const uint32_t tbase = *tslot;
-  if (tid == 0) fd_stamp(p, 1);
   // TMEM columns: [xa: 2 x (32 hi | 32 lo)] [d1: 2 x ND] [mt: H hi | H lo] [d2: 2 x R*ND], ND = N1 or (merged) 2 N1.
   // A tcgen05.mma of this shape costs ~40 cycles whatever its N (TMEM A-operand fetch), and this kernel's steady state was
   // exactly its 96 MMAs per tile; the B operands already hold their hi and lo images back to back with one row-group
@@ -183,7 +170,7 @@ k_fwd_tc(const __grid_constant__ CUtensorMap tmx, const FdTc p) {
             for (int j = 0; j < 4; j++) mma_tf32_ts(d, xa + 32 + 8 * j, dt + (uint64_t)(j * 16), idesc, 1u);
           } else {
             _Pragma("unroll") for (int pass = 0; pass < 3; pass++) {
-              if (pass >= ((p.debug & 2) ? 0 : p.npass)) break;
+              if (pass >= p.npass) break;
               const uint32_t ac = pass == 1 ? xa + 32 : xa;
               const uint64_t dt = (pass == 2 ? d_tl : d_th) + (uint64_t)(c * 64);     // 32 K elements = 8 chunks of 128 B
 #pragma unroll
@@ -244,7 +231,6 @@ k_fwd_tc(const __grid_constant__ CUtensorMap tmx, const FdTc p) {
     for (long g = grp; g < total; g += 2) {
       const int s = (int)(g % p.S);
       mbar_wait(&full[s], (uint32_t)(g / p.S) & 1u);
-      if (g == 0 && tid == 0) fd_stamp(p, 2);
       const uint8_t* row = smem + L.stages + (size_t)s * 16384 + (size_t)m * 128;
       float hi[32], lo[32];
 #pragma unroll
@@ -256,14 +242,11 @@ k_fwd_tc(const __grid_constant__ CUtensorMap tmx, const FdTc p) {
       mbar_wait(&xa_empty[grp], ((uint32_t)(g >> 1) & 1u) ^ 1u);
       tc_fence_after();
       const uint32_t xa = t_xa + lane_base + 64u * grp;
-      if (!(p.debug & 1)) {
-        tmem_st16(xa, hi); tmem_st16(xa + 16, hi + 16);
-        tmem_st16(xa + 32, lo); tmem_st16(xa + 48, lo + 16);
-      }
+      tmem_st16(xa, hi); tmem_st16(xa + 16, hi + 16);
+      tmem_st16(xa + 32, lo); tmem_st16(xa + 48, lo + 16);
       tmem_st_wait();
       tc_fence_before();
       mbar_arrive(&xa_full[grp]);
-      if (g == 0 && tid == 0) fd_stamp(p, 3);
     }
   } else if (warp >= 12) {
     // ===================== hand-over: D1 (TMEM) -> hi/lo K-major B operand of stage 2 (shared memory) =====================
@@ -292,12 +275,10 @@ k_fwd_tc(const __grid_constant__ CUtensorMap tmx, const FdTc p) {
       tmem_st_wait();
       tc_fence_before();
       mbar_arrive(mt_ready);
-      if (tid == 12 * 32) fd_stamp(p, 4);
     }
     for (int it = 0; it < ntiles; it++) {
       const int db = it & 1;
       mbar_wait(&d1_full[db], (uint32_t)(it >> 1) & 1u);
-      if (it == 0 && tid == 12 * 32) fd_stamp(p, 5);
       tc_fence_after();
       float v[32];
 #pragma unroll
@@ -325,7 +306,7 @@ k_fwd_tc(const __grid_constant__ CUtensorMap tmx, const FdTc p) {
       const uint32_t koff = (uint32_t)(m >> 2) * kB2Lbo + (uint32_t)(m & 3) * 4;
 #pragma unroll
       for (int q = 0; q < 32; q++) {
-        if (q < N1 && !(p.debug & 4)) {
+        if (q < N1) {
           const uint32_t off = (uint32_t)(q >> 3) * kB2Sbo + (uint32_t)(q & 7) * 16 + koff;
           *(float*)(bh + off) = v[q];
           *(float*)(bl + off) = tf32_lo(v[q]);
@@ -333,7 +314,6 @@ k_fwd_tc(const __grid_constant__ CUtensorMap tmx, const FdTc p) {
       }
       fence_proxy_async();
       mbar_arrive(&b2_full[db]);
-      if (it == 0 && tid == 12 * 32) fd_stamp(p, 6);
     }
   } else {
     // ===================== spectrum write-out (warps 8, 9 = TMEM lanes 0-31 Re rows, 32-63 Im rows) =====================
@@ -343,7 +323,6 @@ k_fwd_tc(const __grid_constant__ CUtensorMap tmx, const FdTc p) {
       const long tile = t_first + it;
       float* xch = (float*)(smem + L.xch) + (size_t)db * R * 32 * N1;
       mbar_wait(&d2_full[db], (uint32_t)(it >> 1) & 1u);
-      if (it == 0 && tid == 256) fd_stamp(p, 7);
       tc_fence_after();
       if (quad == 1) {
         // Im rows: lane kx holds sum_h Im M[h, kx] * (A re | A im)
@@ -416,19 +395,13 @@ k_fwd_tc(const __grid_constant__ CUtensorMap tmx, const FdTc p) {
         mbar_arrive(&d2_empty[db]);
       }
     }
-    if (tid == 256) fd_stamp(p, 8);
   }
   tc_fence_before();
   __syncthreads();
   if (warp == 11) tmem_dealloc(tbase, 512);
-  if (tid == 0) fd_stamp(p, 9);
 }
 
 }  // namespace
-
-extern "C" int b2no_debug_fd_ts(unsigned long long* host16) {
-  return (int)cudaMemcpyFromSymbol(host16, g_fd_ts, sizeof(unsigned long long) * 16);
-}
 
 void b2no_tc_count_launch();
 
@@ -445,11 +418,8 @@ int b2no_tc_dft_forward(const b2no_plan* plan, int which, const float* x, float*
   const long rows = planes * tf.H;
   p.tiles = (rows + 127) / 128;
   p.tb = tf.tb; p.mimg = tf.mimg; p.spec = spec; p.layout = plan->g.spec_layout;
-  B2NO_ENV_ONCE(env_debug, "B2NO_FD_DEBUG", 0);
-  B2NO_ENV_ONCE(env_merge, "B2NO_FD_MERGE", 1);
-  p.debug = env_debug;
   p.npass = b2no_tc_passes();
-  p.MG = (128u + 4u * p.N1 + 2u * p.H + 4u * p.R * p.N1 <= 512u && env_merge != 0 && p.npass == 3) ? 1 : 0;
+  p.MG = (128u + 4u * p.N1 + 2u * p.H + 4u * p.R * p.N1 <= 512u && p.npass == 3) ? 1 : 0;
   if (!p.MG && 128u + 2u * p.N1 + 2u * p.H + 2u * p.R * p.N1 > 512u) return 1;
   int dev = 0, max_smem = 0;
   B2NO_CHECK_CUDA(cudaGetDevice(&dev));

@@ -46,20 +46,7 @@ struct HeadBwd {
   const float* w1; const float* b1; const float* w2; const float* g; const float* dz;
   float* gx; float* partial;
   int nsum;                                      // floats per partial row: H*Ci + 2H + 1
-  int skip;                                      // ablation mask (B2NO_HB_SKIP, timing experiments only): 1 G1, 2 G3, 4 G2, 8 math, 16 gx stores, 32 Fs stores, 64 F TMEM stores
 };
-
-// -DB2NO_HB_STAMPS: CTA 0 records clock64() at the hand-over points of its first 64 steps (scripts/hb_stamps.py)
-#ifdef B2NO_HB_STAMPS
-__device__ long long* g_hb_stamps = nullptr;
-#define HB_STAMP(role, idx, ev)                                                                              \
-  do {                                                                                                       \
-    if (g_hb_stamps && blockIdx.x == 0 && (idx) < 64 && (threadIdx.x & 31) == 0)                             \
-      g_hb_stamps[((role) * 64 + (idx)) * 8 + (ev)] = clock64();                                             \
-  } while (0)
-#else
-#define HB_STAMP(role, idx, ev) do { } while (0)
-#endif
 
 // act'(z) of the layer below, out of line: the switch over the activations would otherwise be unrolled 32 times
 __device__ __noinline__ float hb_act_grad(float z, int act) { return b2no_act_grad(z, act); }
@@ -204,34 +191,29 @@ k_head_bwd(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUte
       mbar_wait(f_full, (uint32_t)pn & 1u);
       if (ps == 0) mbar_wait(xk_full, (uint32_t)pit & 1u);
       tc_fence_after();
-      HB_STAMP(0, pn, 2);
       if (elect_one()) {
         const uint32_t d3 = t_d3 + (uint32_t)(b * 2 * Cq);
         const uint64_t dxk = d_xk + (uint64_t)(q * 16 * (kHbLbo / 16));        // 64 px = 16 K-chunks of 4
         const uint32_t first = (pit == 0 && q == 0) ? 0u : 1u;
-        if (!(p.skip & 2))
 #pragma unroll
         for (int k = 0; k < 8; k++) mma_tf32_ts(d3, t_f + 8 * k, dxk + (uint64_t)(k * (2 * kHbLbo / 16)), id_n2, (k > 0) ? 1u : first);
-        if (lo_pass && !(p.skip & 2)) {
+        if (lo_pass) {
 #pragma unroll
           for (int k = 0; k < 8; k++) mma_tf32_ts(d3, t_f + 64 + 8 * k, dxk + (uint64_t)(k * (2 * kHbLbo / 16)), id_n1, 1u);
         }
       }
       __syncwarp();
-      HB_STAMP(0, pn, 3);
       if (b == 0) {
         const long qc = (long)pit * 2 + q;
         mbar_wait(d2_empty, ((uint32_t)qc & 1u) ^ 1u);
         tc_fence_after();
       }
-      HB_STAMP(0, pn, 4);
       if (elect_one()) {
         const uint64_t dw = d_wt + (uint64_t)(b * 32 * (128 / 16));             // 128 j = 32 K-chunks of 4
-        if (!(p.skip & 4))
 #pragma unroll
         for (int k = 0; k < 16; k++)
           mma_tf32_ss(t_d2, d_fsh + (uint64_t)(k * (2 * kHbLbo / 16)), dw + (uint64_t)(k * 16), id_g2h, (b > 0 || k > 0) ? 1u : 0u);
-        if (lo_pass && !(p.skip & 4)) {
+        if (lo_pass) {
 #pragma unroll
           for (int k = 0; k < 16; k++)
             mma_tf32_ss(t_d2, d_fsl + (uint64_t)(k * (2 * kHbLbo / 16)), dw + (uint64_t)(k * 16), id_g2l, 1u);
@@ -241,7 +223,6 @@ k_head_bwd(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUte
         if (ps == NS - 1) mma_commit(xk_empty);
       }
       __syncwarp();
-      HB_STAMP(0, pn, 5);
     };
     // software pipeline over the steps of this CTA: G1 of step n is issued before G3 / G2 of step n - 1 (one call site each)
     const long nsteps = (long)(t_end - t_first) * NS;
@@ -252,12 +233,11 @@ k_head_bwd(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUte
         if (s == 0) { mbar_wait(xt_full, (uint32_t)it & 1u); tc_fence_after(); }
         mbar_wait(d1_empty, ((uint32_t)n & 1u) ^ 1u);
         tc_fence_after();
-        HB_STAMP(0, n, 0);
         if (elect_one()) {
           const uint64_t qoff = (uint64_t)(q * 8 * (sbo_xt / 16));               // 64 px rows = 8 row groups
           uint32_t acc = 0;
           _Pragma("unroll") for (int pass = 0; pass < 3; pass++) {
-            if (pass >= p.npass || (p.skip & 1)) break;
+            if (pass >= p.npass) break;
             const uint32_t a = t_w + (uint32_t)(b * 2 * Cq) + (pass == 1 ? (uint32_t)Cq : 0u);
             const uint64_t dx = (pass == 2 ? d_xtl : d_xth) + qoff;
             _Pragma("unroll") for (int k = 0; k < k1; k++) { mma_tf32_ts(t_d1, a + 8 * k, dx + (uint64_t)(k * 16), id_g1, acc); acc = 1; }
@@ -266,7 +246,6 @@ k_head_bwd(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUte
           if (s == NS - 1) mma_commit(xt_empty);
         }
         __syncwarp();
-        HB_STAMP(0, n, 1);
       }
       if (n > 0) {
         const int ps = s > 0 ? s - 1 : NS - 1;
@@ -326,7 +305,7 @@ k_head_bwd(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUte
         }
         fence_proxy_async();
         asm volatile("bar.sync 2, 128;" ::: "memory");
-        if (warp == 2 && lane == 0 && !(p.skip & 16)) {
+        if (warp == 2 && lane == 0) {
           tma_store_3d(&tmg, smem + L.gxb, pxc, c0, bimg);                      // channels >= Ci are clipped by the tensor map
           tma_store_commit();
         }
@@ -336,9 +315,7 @@ k_head_bwd(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUte
     int it = 0;
     for (int tile = t_first; tile < t_end; tile++, it++) {
       mbar_wait(raw_full, (uint32_t)it & 1u);
-      if (warp == 2) HB_STAMP(2, it, 0);
       mbar_wait(xt_empty, ((uint32_t)it & 1u) ^ 1u);
-      if (warp == 2) HB_STAMP(2, it, 1);
       // the raw tile is read twice (8 channels at a time) instead of being held in 32 registers across the two waits
       for (int c0 = 0; c0 < Cq; c0 += 8) {
         float v[8];
@@ -353,10 +330,8 @@ k_head_bwd(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUte
         }
       }
       fence_proxy_async();
-      if (warp == 2) HB_STAMP(2, it, 2);
       warp_arrive(xt_full);
       mbar_wait(xk_empty, ((uint32_t)it & 1u) ^ 1u);
-      if (warp == 2) HB_STAMP(2, it, 3);
       for (int c0 = 0; c0 < Cq; c0 += 8) {
         float v[8];
 #pragma unroll
@@ -369,7 +344,6 @@ k_head_bwd(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUte
         }
       }
       fence_proxy_async();
-      if (warp == 2) HB_STAMP(2, it, 4);
       warp_arrive2(raw_empty, xk_full);
       if (it > 0) gx_epilogue((long)it * cpt - 1, tile - 1, cpt - 1);           // closed by the last step of the previous tile
       gx_epilogue((long)it * cpt, tile, 0);
@@ -402,7 +376,6 @@ k_head_bwd(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUte
         const int q = NB == 2 ? (s >> 1) : s, b = NB == 2 ? (s & 1) : 0;
         mbar_wait(d1_full, (uint32_t)n & 1u);
         tc_fence_after();
-        if (warp == 6) HB_STAMP(1, n, 0);
         float v[16], gv[16];
         tmem_ld16(t_d1 + lane_base + (uint32_t)(16 * part), v);
 #pragma unroll
@@ -410,15 +383,13 @@ k_head_bwd(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUte
         tmem_ld_wait();
         tc_fence_before();
         warp_arrive(d1_empty);
-        if (warp == 6) HB_STAMP(1, n, 1);
         if (b == 0) {
 #pragma unroll
           for (int i = 0; i < 16; i += 2) gsum = __fadd2_rn(gsum, make_float2(gv[i], gv[i + 1]));
         }
         const float b1j = b == 0 ? b1r[0] : b1r[1], w2j = b == 0 ? w2r[0] : w2r[1];
         float2 dw2v = b == 0 ? dw2a[0] : dw2a[1], dsv = b == 0 ? dsa[0] : dsa[1];
-        if (p.skip & 8) {
-        } else if (GELU) {
+        if (GELU) {
           float2* v2 = reinterpret_cast<float2*>(v);
           const float2* g2 = reinterpret_cast<const float2*>(gv);
           const float2 bb = b2no_f2(b1j), ww = b2no_f2(w2j);
@@ -443,21 +414,18 @@ k_head_bwd(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUte
         }
         if (b == 0) { dw2a[0] = dw2v; dsa[0] = dsv; } else { dw2a[1] = dw2v; dsa[1] = dsv; }
         // F of the previous step must have been consumed by its G3 / G2
-        if (warp == 6) HB_STAMP(1, n, 2);
         mbar_wait(f_empty, ((uint32_t)n & 1u) ^ 1u);
         tc_fence_after();
-        if (warp == 6) HB_STAMP(1, n, 3);
-        if (!(p.skip & 64)) tmem_st16(t_f + lane_base + (uint32_t)(16 * part), v);
+        tmem_st16(t_f + lane_base + (uint32_t)(16 * part), v);
 #pragma unroll
         for (int h = 0; h < 2; h++) {
           float fl[8];
 #pragma unroll
           for (int i = 0; i < 8; i++) fl[i] = v[8 * h + i] - tf32_trunc(v[8 * h + i]);     // exact; the tensor core reads its top 19 bits
-          if (!(p.skip & 64)) tmem_st8(t_f + lane_base + 64u + (uint32_t)(16 * part + 8 * h), fl);
+          tmem_st8(t_f + lane_base + 64u + (uint32_t)(16 * part + 8 * h), fl);
 #pragma unroll
           for (int i = 0; i < 8; i++) {
             const uint32_t off = (uint32_t)h * kHbSbo + (uint32_t)i * 16;
-            if (p.skip & 32) continue;
             sts_f32(fs_base + off, v[8 * h + i]);
             sts_f32(fs_base + L.fs_img + off, fl[i]);
           }
@@ -465,9 +433,7 @@ k_head_bwd(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUte
         tmem_st_wait();
         fence_proxy_async();
         tc_fence_before();
-        if (warp == 6) HB_STAMP(1, n, 4);
         warp_arrive(f_full);
-        if (warp == 6) HB_STAMP(1, n, 5);
       }
     }
     // ---- read-out: dW1 from D3, dw2 / db1 from the register sums (column parts combined through shared memory) ----
@@ -568,12 +534,6 @@ bool hb_shape_ok(int ci, int hidden, long pixels) {
 
 void b2no_tc_count_launch();
 
-#ifdef B2NO_HB_STAMPS
-extern "C" int b2no_debug_head_bwd_stamps(long long* buf) {
-  return (int)cudaMemcpyToSymbol(g_hb_stamps, &buf, sizeof(buf));
-}
-#endif
-
 extern "C" int b2no_mlp_head_bwd_fused_supported(int ci, int hidden, int64_t pixels) {
   return hb_shape_ok(ci, hidden, (long)pixels) ? 1 : 0;
 }
@@ -601,8 +561,6 @@ extern "C" int b2no_mlp_head_bwd_fused(const float* x, const float* w1, const fl
   if (tiles >= (1L << 30)) return B2NO_E_UNSUPPORTED;
   p.tiles = (int)tiles;
   p.nsum = hidden * ci + 2 * hidden + 1;
-  B2NO_ENV_ONCE(hb_skip, "B2NO_HB_SKIP", 0);
-  p.skip = hb_skip;
   int grid = p.tiles < b2no_sm_count() ? p.tiles : b2no_sm_count();
   p.tiles_per_cta = (p.tiles + grid - 1) / grid;
   grid = (p.tiles + p.tiles_per_cta - 1) / p.tiles_per_cta;

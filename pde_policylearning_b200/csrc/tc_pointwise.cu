@@ -27,7 +27,6 @@
 //               left the issue slots half empty), tcgen05.ld -> bias/act -> coalesced global stores;
 //               two TMEM accumulators so the MMAs of tile i+1 overlap the epilogue of tile i.  MODE 3 fetches the
 //               saved pre-activations of the NEXT tile before it waits for the current accumulator.
-#include <stdlib.h>
 #include <string.h>
 
 #include "common.cuh"
@@ -58,7 +57,6 @@ struct PwTc {
   long mul_bs, gate_bs;   // floats between consecutive samples of mul / gate_z
   float* preact; float* y;
   int act, dact;
-  int debug;          // bit0 no stores, bit1 no MMAs
   int npass;          // 3: 3xTF32, 1: single-pass TF32 (hi * hi only)
   // 3-D mode (zlen > 0): rows of the last dim have zlen points, a 128-pixel tile touches up to R = 127 / zlen + 2 of them.
   // The last-stage operand T[pixel, (row slot, q)] then depends on where the tile starts, so the converter warps build it
@@ -216,7 +214,6 @@ k_pw_tc(const __grid_constant__ CUtensorMap tm1, const __grid_constant__ CUtenso
       const uint64_t d_w2h = smem_desc(sbase + L.w2h, 128, (p.C2p / 4) * 128, LAYOUT_NONE);
       const uint64_t d_w2l = smem_desc(sbase + L.w2l, 128, (p.C2p / 4) * 128, LAYOUT_NONE);
       const uint32_t lbo_a = (uint32_t)(p.Np / 8) * 128;
-      const bool nomma = (p.debug & 2) != 0;
       int it = 0;
       for (long tile = t_first; tile < t_end; tile++, it++) {
         const int s = it % p.S;
@@ -233,7 +230,7 @@ k_pw_tc(const __grid_constant__ CUtensorMap tm1, const __grid_constant__ CUtenso
         const uint32_t d = tbase + (uint32_t)a * p.Np;
         const uint32_t xa = a_base + (uint32_t)xi * a_width;
         uint32_t acc = 0;
-        if (!nomma && elect_one()) {
+        if (elect_one()) {
           _Pragma("unroll") for (int pass = 0; pass < 3; pass++) {
             if (pass >= p.npass) break;   // compile-time trip count (descriptors stay folded); 1-pass mode leaves early
             const uint32_t ac = pass == 1 ? xa + p.C1p : xa;
@@ -372,7 +369,6 @@ k_pw_tc(const __grid_constant__ CUtensorMap tm1, const __grid_constant__ CUtenso
     const int t = quad * 32 + lane;
     const uint32_t lane_base = (uint32_t)(quad * 32) << 16;
     const uint32_t sbias = smem_u32(smem) + L.bias;
-    const bool nostore = (p.debug & 1) != 0;
     // MODE 3: the saved pre-activations of the layer below arrive through the TMA ring (dz tile [Cz x 128 px] in the
     // stage, S tiles ahead of their use); with one pass per tile (Co <= 32) the thread takes its 8 values and releases the
     // stage right away, otherwise it reads them pass by pass and releases the stage at the end of the tile.  (Fetching
@@ -423,7 +419,7 @@ k_pw_tc(const __grid_constant__ CUtensorMap tm1, const __grid_constant__ CUtenso
               const float z = v[j] + lds_f32(sbias + (uint32_t)(c0 + j) * 4u) + av[j];
               if (p.preact) p.preact[idx] = z;
               const float r = fmaf(1.0f - gzv[j], ghv[j], epi_value<0>(z, mv[j], dv[j], p.act, p.dact));
-              if (!nostore) p.y[idx] = r;
+              p.y[idx] = r;
             }
           }
         } else {
@@ -470,11 +466,9 @@ k_pw_tc(const __grid_constant__ CUtensorMap tm1, const __grid_constant__ CUtenso
 #pragma unroll
             for (int j = 0; j < kCW; j++) v[j] *= dv[j];
           }
-          if (!nostore) {
 #pragma unroll
-            for (int j = 0; j < kCW; j++)
-              if (c0 + j < p.Co) yp[(size_t)j * p.P] = v[j];
-          }
+          for (int j = 0; j < kCW; j++)
+            if (c0 + j < p.Co) yp[(size_t)j * p.P] = v[j];
         }
       }
       tc_fence_before();
@@ -604,8 +598,6 @@ int g_tc_npass = 3;
 bool b2no_tc_available() {
   if (g_tc_state < 0) {
     int on = 1;
-    const char* e = getenv("B2NO_DISABLE_TC");
-    if (e && e[0] && e[0] != '0') on = 0;
     int dev = 0, major = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev) != cudaSuccess ||
         major != 10)
@@ -772,8 +764,6 @@ int b2no_tc_pointwise(const b2no_plan* plan, int which, const float* spec, float
   long grid = p.tiles < b2no_sm_count() ? p.tiles : b2no_sm_count();
   p.tiles_per_cta = (p.tiles + grid - 1) / grid;
   grid = (p.tiles + p.tiles_per_cta - 1) / p.tiles_per_cta;
-  B2NO_ENV_ONCE(env_debug, "B2NO_TC_DEBUG", 0);
-  p.debug = env_debug;
   p.npass = b2no_tc_passes();
 #define LAUNCH(M)                                                                                                  \
   do {                                                                                                             \

@@ -25,14 +25,13 @@ using namespace tc;
 namespace {
 
 constexpr int kThreadsWg = 320;  // warps 0-3 converter group A (+ final read-out), 4-7 converter group B, 8 TMA, 9 MMA
+constexpr int kWgSlots = 2;      // A-ring slots (TMEM operand + lo copy), one per converter group
 
 struct WgTc {
   int Co, Cop, Ci, Cip, TP, SUB, nb, S, mblocks;   // TP = pixels per TMA stage, SUB = pixels per MMA chunk (A ring slot)
-  int NS;                                          // A-ring slots (TMEM operand + lo copy): 4 when one M block, else 2
   int tiles_per_img;
   long tiles, tiles_per_cta;
   float* partial;
-  int debug;    // ablation (B2NO_WG_DEBUG): 1 no X-lo pass, 2 no G conversion, 4 no MMAs
   int npass;    // 3: 3xTF32, 1: single-pass TF32 (G_hi x X_hi only, accumulator columns [0, Cip))
 };
 
@@ -48,29 +47,13 @@ __host__ __device__ inline WgLayout wg_layout(const WgTc& p) {
   L.stage_bytes = (L.gbytes + L.xbytes + 1023u) & ~1023u;
   L.dbs = L.stage_bytes * p.S;
   L.bars = L.dbs + 2u * p.mblocks * 128 * 4;
-  L.total = L.bars + 8 * (2 * p.S + 2 * p.NS + 1) + 16 + 1024;
+  L.total = L.bars + 8 * (2 * p.S + 2 * kWgSlots + 1) + 16 + 1024;
   return L;
 }
 
 // TMEM columns: A operand ring [slot][M-block][hi SUB | lo SUB], then the accumulators [M-block][2 Cip]
 // (columns [0, Cip): G_hi X_hi + G_lo X_hi, columns [Cip, 2 Cip): G_hi X_lo; added at read-out)
-__host__ __device__ inline uint32_t wg_tmem_cols(const WgTc& p) { return 2u * p.NS * p.SUB * p.mblocks + 2u * p.mblocks * p.Cip; }
-
-// debug: %globaltimer stamps of CTA 0 for its first 16 chunks (B2NO_WG_DEBUG & 16), read back with b2no_debug_wg_ts.
-// slot = chunk * 8 + {0 slot free seen, 1 lo copy done, 2 conversion issued, 3 TMEM stores complete, 4 MMA warp saw a_full,
-// 5 MMAs issued + committed, 6 stage full seen (converter), 7 unused}
-// The stamps sit on the hand-over path (every instruction there shows in the launch time), so they are compiled in only
-// with -DB2NO_WG_STAMPS (scripts/wg_ts.py explains how).
-__device__ unsigned long long g_wg_ts[128];
-__device__ __forceinline__ void wg_stamp(const WgTc& p, long n, int what) {
-#ifdef B2NO_WG_STAMPS
-  if ((p.debug & 16) && blockIdx.x == 0 && n < 16) {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-    g_wg_ts[n * 8 + what] = t;
-  }
-#endif
-}
+__host__ __device__ inline uint32_t wg_tmem_cols(const WgTc& p) { return 2u * kWgSlots * p.SUB * p.mblocks + 2u * p.mblocks * p.Cip; }
 
 __global__ void __launch_bounds__(kThreadsWg, 1)
 k_wgrad_tc(const __grid_constant__ CUtensorMap tmg, const __grid_constant__ CUtensorMap tmx, const WgTc p) {
@@ -80,8 +63,8 @@ k_wgrad_tc(const __grid_constant__ CUtensorMap tmg, const __grid_constant__ CUte
   uint64_t* full = (uint64_t*)(smem + L.bars);
   uint64_t* empty = full + p.S;
   uint64_t* a_full = empty + p.S;
-  uint64_t* a_empty = a_full + p.NS;
-  uint64_t* done = a_empty + p.NS;
+  uint64_t* a_empty = a_full + kWgSlots;
+  uint64_t* done = a_empty + kWgSlots;
   uint32_t* tslot = (uint32_t*)(done + 1);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int NW = p.Cip, TP = p.TP;
@@ -90,7 +73,7 @@ k_wgrad_tc(const __grid_constant__ CUtensorMap tmg, const __grid_constant__ CUte
 
   if (tid == 0) {
     for (int s = 0; s < p.S; s++) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
-    for (int a = 0; a < p.NS; a++) { mbar_init(&a_full[a], 128); mbar_init(&a_empty[a], 1); }
+    for (int a = 0; a < kWgSlots; a++) { mbar_init(&a_full[a], 128); mbar_init(&a_empty[a], 1); }
     mbar_init(done, 1);
     fence_barrier_init();
   }
@@ -102,8 +85,7 @@ k_wgrad_tc(const __grid_constant__ CUtensorMap tmg, const __grid_constant__ CUte
   tc_fence_after();
   const uint32_t tbase = *tslot;
   const int SUB = p.SUB, nsub = TP / SUB, nbs = SUB / 32;
-  const uint32_t t_acc = tbase + 2u * p.NS * SUB * p.mblocks;
-  const int NS = p.NS;   // 2 or 3
+  const uint32_t t_acc = tbase + 2u * kWgSlots * SUB * p.mblocks;
   const long t_first = (long)blockIdx.x * p.tiles_per_cta;
   const long t_end = t_first + p.tiles_per_cta < p.tiles ? t_first + p.tiles_per_cta : p.tiles;
 
@@ -140,14 +122,13 @@ k_wgrad_tc(const __grid_constant__ CUtensorMap tmg, const __grid_constant__ CUte
       const uint32_t ph = (uint32_t)(it / p.S) & 1u;
       mbar_wait(&full[s], ph);
       for (int sub = 0; sub < nsub; sub++, n++) {
-        const uint32_t un = (uint32_t)n, uq = NS == 3 ? un / 3u : un >> 1;   // 32-bit: a 64-bit division here cost 15 us per launch
-        const int ab = (int)(un - uq * (uint32_t)NS);
+        const uint32_t un = (uint32_t)n, uq = un / kWgSlots;   // 32-bit: a 64-bit division here cost 15 us per launch
+        const int ab = (int)(un % kWgSlots);
         mbar_wait(&a_full[ab], uq & 1u);
         tc_fence_after();
-        if (lane == 0) wg_stamp(p, n, 4);
         if (elect_one()) {
           const uint32_t st = sbase + (uint32_t)s * L.stage_bytes;
-          for (int mb = 0; mb < ((p.debug & 4) ? 0 : p.mblocks); mb++) {
+          for (int mb = 0; mb < p.mblocks; mb++) {
             const uint32_t d = t_acc + (uint32_t)(mb * 2 * NW);
             const uint32_t a0 = tbase + (uint32_t)((ab * p.mblocks + mb) * 2 * SUB);
             uint32_t a2 = acc;
@@ -170,15 +151,14 @@ k_wgrad_tc(const __grid_constant__ CUtensorMap tmg, const __grid_constant__ CUte
         }
         acc = 1;
         __syncwarp();
-        if (lane == 0) wg_stamp(p, n, 5);
       }
     }
     if (elect_one()) mma_commit(done);
     __syncwarp();
   } else {
     // ===================== converter: X lo in shared memory; G rows -> TMEM A operand (thread = channel row) =====================
-    // two groups of four warps alternate over the sub-chunks (chunk n -> group n % 2, ring slot n % NS), so conversion of
-    // chunk n+1 overlaps the MMAs of chunk n; with NS = 4 a group also starts chunk n+2 before the MMAs of chunk n finish
+    // two groups of four warps alternate over the sub-chunks (chunk n -> group n % 2 and ring slot n % 2), so conversion of
+    // chunk n+1 overlaps the MMAs of chunk n
     const int grp = warp >> 2;
     const int ct = tid & 127;
     const int quad = warp & 3;
@@ -191,7 +171,6 @@ k_wgrad_tc(const __grid_constant__ CUtensorMap tmg, const __grid_constant__ CUte
       const int s = it % p.S;
       const uint32_t ph = (uint32_t)(it / p.S) & 1u;
       mbar_wait(&full[s], ph);
-      if (m == 0 && grp == 0) wg_stamp(p, n, 6);
       uint8_t* st = smem + (size_t)s * L.stage_bytes;
       for (int sub = 0; sub < nsub; sub++, n++) {
         // (measured and rejected: BOTH groups converting every chunk, one box each: 96 vs 80 us -- every chunk then
@@ -204,7 +183,7 @@ k_wgrad_tc(const __grid_constant__ CUtensorMap tmg, const __grid_constant__ CUte
           const int first_idle = (p.mblocks == 1) ? ((p.Cop + 31) >> 5) : 4;      // quads >= first_idle hold only pad rows
           const int nidle = 4 - first_idle;
           const bool copier = nidle == 0 || quad >= first_idle;
-          if (copier && !(p.debug & 1)) {
+          if (copier) {
             const int cthreads = nidle == 0 ? 128 : nidle * 32;
             const int cid = nidle == 0 ? ct : (quad - first_idle) * 32 + lane;
             const uint32_t per_box = (uint32_t)NW * 128 / 16;
@@ -218,15 +197,13 @@ k_wgrad_tc(const __grid_constant__ CUtensorMap tmg, const __grid_constant__ CUte
             }
           }
         }
-        const uint32_t un = (uint32_t)n, uq = NS == 3 ? un / 3u : un >> 1;
-        const int ab = (int)(un - uq * (uint32_t)NS);
+        const uint32_t un = (uint32_t)n, uq = un / kWgSlots;
+        const int ab = (int)(un % kWgSlots);
         mbar_wait(&a_empty[ab], (uq & 1u) ^ 1u);                     // MMAs of this slot's previous chunk are complete
         tc_fence_after();
-        if (m == 0) wg_stamp(p, n, 0);
-        if (m == 0) wg_stamp(p, n, 1);
 #pragma unroll
         for (int mb = 0; mb < 3; mb++) {
-          if (mb >= ((p.debug & 2) ? 0 : p.mblocks)) break;
+          if (mb >= p.mblocks) break;
           const int row = mb * 128 + m;
           const uint32_t a0 = tbase + lane_base + (uint32_t)((ab * p.mblocks + mb) * 2 * SUB);
           // tcgen05.st is warp-collective (.sync.aligned): the branch must be warp-uniform, so a warp that owns at least
@@ -254,7 +231,7 @@ k_wgrad_tc(const __grid_constant__ CUtensorMap tmg, const __grid_constant__ CUte
               tmem_st16(a0 + (uint32_t)(j * 32), hi); tmem_st16(a0 + (uint32_t)(j * 32 + 16), hi + 16);
               tmem_st16(a0 + (uint32_t)(SUB + j * 32), lo); tmem_st16(a0 + (uint32_t)(SUB + j * 32 + 16), lo + 16);
             }
-          } else if (n < NS) {
+          } else if (n < kWgSlots) {
             // pad rows (>= Cop) of an M block: zeroed once per ring slot, never written again
             float z[16];
 #pragma unroll
@@ -262,11 +239,9 @@ k_wgrad_tc(const __grid_constant__ CUtensorMap tmg, const __grid_constant__ CUte
             for (int c = 0; c < 2 * SUB; c += 16) tmem_st16(a0 + (uint32_t)c, z);
           }
         }
-        if (m == 0) wg_stamp(p, n, 2);
         tmem_st_wait();
         tc_fence_before();
         fence_proxy_async();
-        if (m == 0) wg_stamp(p, n, 3);
         mbar_arrive(&a_full[ab]);
       }
     }
@@ -314,10 +289,6 @@ k_wgrad_tc(const __grid_constant__ CUtensorMap tmg, const __grid_constant__ CUte
 
 void b2no_tc_count_launch();
 
-extern "C" int b2no_debug_wg_ts(unsigned long long* host128) {
-  return (int)cudaMemcpyFromSymbol(host128, g_wg_ts, sizeof(unsigned long long) * 128);
-}
-
 // Fills `partial` with *nblk per-CTA partials laid out [Co*Ci | Co]; returns 0 on success, 1 if not eligible.
 int b2no_tc_wgrad(const float* g, const float* x, float* partial, int max_blocks, int batch, int ci, int co, long pixels,
                   int* nblk, cudaStream_t st) {
@@ -335,11 +306,8 @@ int b2no_tc_wgrad(const float* g, const float* x, float* partial, int max_blocks
   bool ok = false;
   // two ring slots of 64 px (one M block) / 32 px.  Measured on B200 (cfg2, Co = Ci = 32): four slots of 32 px are SLOWER
   // (155 us vs 87 us) -- the cost is per chunk hand-over (~0.7 us), not per pixel, so chunks are as large as TMEM allows;
-  // a third 64-px slot (B2NO_WG_SLOTS=3) changes nothing (93.6 vs 93.4 us): the converters do not wait for free slots
+  // a third 64-px slot changes nothing (93.6 vs 93.4 us): the converters do not wait for free slots
   p.SUB = p.mblocks == 1 ? 64 : 32;
-  B2NO_ENV_ONCE(env_slots, "B2NO_WG_SLOTS", 2);
-  p.NS = (p.mblocks == 1 && env_slots == 3) ? 3 : 2;
-  if (wg_tmem_cols(p) > 512) p.NS = 2;
   if (p.mblocks > 3 || wg_tmem_cols(p) > 512) return 1;
   // bytes in flight decide an HBM-bound kernel: take the largest tile that still leaves >= 4 stages, else the deepest ring
   for (int pass = 0; pass < 2 && !ok; pass++)
@@ -361,8 +329,6 @@ int b2no_tc_wgrad(const float* g, const float* x, float* partial, int max_blocks
   p.tiles_per_cta = (p.tiles + grid - 1) / grid;
   grid = (p.tiles + p.tiles_per_cta - 1) / p.tiles_per_cta;
   p.partial = partial;
-  B2NO_ENV_ONCE(env_debug, "B2NO_WG_DEBUG", 0);
-  p.debug = env_debug;
   p.npass = b2no_tc_passes();
   CUtensorMap tmg, tmx;
   {

@@ -12,6 +12,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def test_library_exports_every_declared_symbol():
+    import subprocess
     from pde_policylearning_b200 import _lib
     if not os.path.exists(_lib.LIB_PATH):
         _lib.build()
@@ -21,6 +22,9 @@ def test_library_exports_every_declared_symbol():
     L = ctypes.CDLL(_lib.LIB_PATH)
     for name in declared:
         assert hasattr(L, name), f"{name} declared in include/b2no.h but not exported"
+    nm = subprocess.run(["nm", "-D", "--defined-only", _lib.LIB_PATH], check=True, capture_output=True, text=True).stdout
+    defined = set(re.findall(r"\b(b2no_[a-z0-9_]+)$", nm, re.M))
+    assert defined == declared, f"exported, not declared in include/b2no.h: {sorted(defined - declared)}"
     assert set(_lib.EXPORTS) == declared
     assert _lib.lib().b2no_version() == 5
     assert b"bad argument" in _lib.lib().b2no_error_string(-1)
