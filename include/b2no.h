@@ -155,6 +155,17 @@ int b2no_act_bwd(const float* gy, const float* z, float* gz, int64_t n, int act,
 int64_t b2no_pw_wgrad_scratch_floats(int ci, int co);
 int b2no_pw_wgrad(const float* g, const float* x, float* dw, float* db, float* partial, int batch, int ci,
                   int co, int64_t pixels, void* stream);
+/* The dx pass of a 2-D FNO layer and the weight gradient of its 1x1 skip in one pass over the pixel tiles:
+ *   y = b2no_dft_inverse(plan, which, spec, ..., epi)   with epi->pw_x = g (batch, co = epi->pw_ci, pixels)
+ *   dw[o,i] = sum_{b,p} g[b,o,p] x[b,i,p] ;  db[o] = sum_{b,p} g[b,o,p] (db may be NULL)      x = wg_x (batch, wg_ci, pixels)
+ * -- b2no_dft_inverse followed by b2no_pw_wgrad(g, x), without reading g a second time.  partial: scratch of
+ * b2no_pw_wgrad_scratch_floats(wg_ci, co) floats.  Runs on the tensor-core tile kernel only: returns B2NO_E_UNSUPPORTED, having
+ * written nothing, when it cannot (not a 2-D plan, no tensor cores, an epilogue with anything but pw_w / pw_x -- bias, act,
+ * dact_z, a second 1x1 operand --, co > 64, wg_ci > 112, pixels % 128 != 0, misaligned pointers, shared memory too small);
+ * the caller then makes the two calls. */
+int b2no_dft_inverse_wgrad(const b2no_plan* plan, int which, const float* spec, float* y, float* work, int batch, int channels,
+                           int64_t pixels, const b2no_epilogue* epi, const float* wg_x, int wg_ci, float* dw, float* db,
+                           float* partial, void* stream);
 /* fused projection head (tfno.py:34-38; pinobserver.py:230-232 after folding MultiplicativeNet):
  *   out[b,p] = b2 + sum_j w2[j] * gelu( b1[(b),j] + sum_i w1[j,i] x[b,i,p] )      (out_channels == 1)
  * b1 is (hidden) or, when b1_per_sample, (batch, hidden). */

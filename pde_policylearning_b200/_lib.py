@@ -108,6 +108,7 @@ def lib():
     L.b2no_pw_wgrad_scratch_floats.restype = i64
     L.b2no_pw_wgrad_scratch_floats.argtypes = [i32, i32]
     L.b2no_pw_wgrad.argtypes = [vp, vp, vp, vp, vp, i32, i32, i32, i64, vp]
+    L.b2no_dft_inverse_wgrad.argtypes = [vp, i32, vp, vp, vp, i32, i32, i64, C.POINTER(Epilogue), vp, i32, vp, vp, vp, vp]
     L.b2no_mlp_head_fwd.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, i32, i64, i32, i32, vp]
     L.b2no_mlp_head_bwd_supported.argtypes = [i32, i32, i64]
     L.b2no_mlp_head_bwd_scratch_floats.restype = i64
@@ -144,7 +145,7 @@ EXPORTS = [
     "b2no_plan_create", "b2no_plan_destroy", "b2no_plan_kept", "b2no_plan_layout_supported", "b2no_plan_workspace_floats",
     "b2no_set_tensor_core_mode", "b2no_set_precision", "b2no_tensor_core_launches", "b2no_kernel_launches",
     "b2no_dft_forward", "b2no_dft_inverse", "b2no_mix", "b2no_mix_dw",
-    "b2no_act_bwd", "b2no_pw_wgrad_scratch_floats", "b2no_pw_wgrad", "b2no_mlp_head_fwd", "b2no_mlp_head_bwd_scratch_floats", "b2no_mlp_head_bwd_supported", "b2no_mlp_head_bwd",
+    "b2no_act_bwd", "b2no_pw_wgrad_scratch_floats", "b2no_pw_wgrad", "b2no_dft_inverse_wgrad", "b2no_mlp_head_fwd", "b2no_mlp_head_bwd_scratch_floats", "b2no_mlp_head_bwd_supported", "b2no_mlp_head_bwd",
     "b2no_mlp_head_bwd_fused_scratch_floats", "b2no_mlp_head_bwd_fused_supported", "b2no_mlp_head_bwd_fused",
     "b2no_rno_gate_fwd", "b2no_rno_gate_bwd", "b2no_rno_cell_bwd", "b2no_rno_reset_bwd", "b2no_rel_l2_sums", "b2no_rel_l2_bwd",
     "b2no_rel_l2_finish", "b2no_rel_l2_bwd_g", "b2no_adam_step", "b2no_gather_segments",

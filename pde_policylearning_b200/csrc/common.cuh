@@ -31,8 +31,16 @@ int b2no_tc_mlp_fwd(const float* x, const float* w1, const float* b1, const floa
                     int ci, int hidden, int co2, long pixels, int b1_per_sample, int act, cudaStream_t st);
 int b2no_tc_wgrad(const float* g, const float* x, float* partial, int max_blocks, int batch, int ci, int co, long pixels,
                   int* nblk, cudaStream_t st);
+// weight-gradient variant of the 2-D dx pass (b2no_dft_inverse_wgrad): dW[o, i] = sum pw_x[b, o, p] x[b, i, p] and
+// db[o] = sum pw_x[b, o, p] into per-CTA partials [Co*Ci | Co] (*nblk of them, summed by k_pw_wgrad_reduce)
+struct b2no_tc_wg {
+  const float* x;
+  int ci;
+  float* partial;
+  int* nblk;
+};
 int b2no_tc_pointwise(const b2no_plan* plan, int which, const float* spec, float* y, float* work, int batch, int channels,
-                      long pixels, const b2no_epilogue* e, cudaStream_t st);
+                      long pixels, const b2no_epilogue* e, cudaStream_t st, const b2no_tc_wg* wg = nullptr);
 
 // operand images for the tensor-core tile kernel (tc_pointwise.cu): the last-dim inverse table as a
 // block-diagonal row-major [128 x Ks] matrix, hi then lo (3xTF32); it becomes a TMEM-resident A operand

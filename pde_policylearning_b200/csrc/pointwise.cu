@@ -251,6 +251,29 @@ extern "C" int b2no_pw_wgrad(const float* g, const float* x, float* dw, float* d
   return 0;
 }
 
+extern "C" int b2no_dft_inverse_wgrad(const b2no_plan* plan, int which, const float* spec, float* y, float* work, int batch,
+                                     int channels, int64_t pixels, const b2no_epilogue* epi, const float* wg_x, int wg_ci,
+                                     float* dw, float* db, float* partial, void* stream) {
+  if (!plan || !spec || !y || !work || !epi || !wg_x || !dw || !partial || batch < 1 || channels < 1 || wg_ci < 1 ||
+      (which != 0 && which != 1))
+    return B2NO_E_ARG;
+  if (!epi->pw_w || !epi->pw_x || epi->pw_ci < 1) return B2NO_E_ARG;
+  if (plan->g.ndim != 2) return B2NO_E_UNSUPPORTED;
+  const int32_t* n = which == 0 ? plan->g.nout : plan->g.nin;
+  const long px = (long)n[0] * n[1];
+  if (pixels > 0 && pixels != px) return B2NO_E_ARG;
+  cudaStream_t st = (cudaStream_t)stream;
+  int nblk = 0;
+  const b2no_tc_wg wg = {wg_x, wg_ci, partial, &nblk};
+  const int rc = b2no_tc_pointwise(plan, which, spec, y, work, batch, channels, px, epi, st, &wg);
+  if (rc == 1) return B2NO_E_UNSUPPORTED;
+  if (rc) return rc;
+  const int co = epi->pw_ci, nw = co * wg_ci + co;
+  k_pw_wgrad_reduce<<<(nw + 31) / 32, 256, 0, st>>>(partial, dw, db, nblk, wg_ci, co);
+  B2NO_LAUNCH_CHECK();
+  return 0;
+}
+
 // ---------------------------------------------------------------------------------------------
 // fused projection head, out_channels == 1: two pixels per thread, W1 in shared memory
 // ---------------------------------------------------------------------------------------------

@@ -64,16 +64,27 @@ struct PwTc {
   int zlen, q2, tz_npad;
   long RPI;           // rows per sample (n0 * n1)
   const float* tz;
+  // Weight-gradient variant (k_pw_tc<MODE, true>, 2-D dx passes): dWp[o, i] = sum_p X1[o, p] XW[i, p], db[o] = sum_p X1[o, p]
+  // over the tiles of the CTA, written as per-CTA partials.  MW = M of those MMAs (64 or 128 >= the 2 C1p rows [X1 hi ; X1 lo];
+  // the rows past them read whatever follows in the stage and land in accumulator rows nobody reads), NW = their N
+  // ([XW hi ; XW lo ; ones], Cxp = XW channels rounded up to 8; the ones block makes db an accumulator column); 0 in the
+  // plain kernel.
+  int MW, NW, Cx, Cxp;
+  float* wpart;
 };
 
 struct PwLayout {
-  uint32_t w1h, w1l, w2h, w2l, bias, tzh, tzl, stages, stage_bytes, x2, ah, al, dz, bars, total;
+  uint32_t w1h, w1l, w2h, w2l, bias, tzh, tzl, stages, stage_bytes, x2, xw, ah, al, dz, bars, total;
 };
 
+// WG (compile-time, so that the plain kernels' code does not depend on the variant): the weight-gradient variant, where X1
+// arrives as four SW128 boxes [32 px x C1p], each followed by its lo copy (2 C1p rows per box), then four XW boxes of NW rows
+template <bool WG>
 __host__ __device__ inline PwLayout pw_layout(const PwTc& p) {
   PwLayout L;
   const uint32_t wb1 = (uint32_t)p.Np * p.C1p * 4, wb2 = (uint32_t)p.Np * p.C2p * 4;
-  const uint32_t xb1 = (uint32_t)p.C1p * 512, xb2 = (uint32_t)p.C2p * 512, ab = (uint32_t)p.Ks * p.Np * 4;
+  const uint32_t xb1 = (uint32_t)p.C1p * (WG ? 1024 : 512), xb2 = (uint32_t)p.C2p * 512;
+  const uint32_t xwb = WG ? (uint32_t)p.NW * 512 : 0u, ab = (uint32_t)p.Ks * p.Np * 4;
   uint32_t o = 0;
   L.w1h = o; o += wb1; L.w1l = o; o += wb1;
   L.w2h = o; o += wb2; L.w2l = o; o += wb2;
@@ -82,20 +93,24 @@ __host__ __device__ inline PwLayout pw_layout(const PwTc& p) {
   L.tzl = o; o += (uint32_t)p.Qp * p.zlen * 4;
   o = (o + 1023u) & ~1023u;
   L.stages = o;
-  L.x2 = xb1; L.ah = xb1 + xb2; L.al = L.ah + ab;
+  L.x2 = xb1; L.xw = xb1 + xb2; L.ah = L.xw + xwb; L.al = L.ah + ab;
   L.dz = (L.al + ab + 127u) & ~127u;
   L.stage_bytes = (L.dz + (uint32_t)p.Cz * 512 + 1023u) & ~1023u;
   o += L.stage_bytes * p.S;
   L.bars = o;
-  o += 8 * (2 * p.S + 8) + 16;
+  o += 8 * (2 * p.S + 8 + (WG ? 1 : 0)) + 16;
   L.total = o + 1024;  // slack for the manual 1024-byte alignment of the dynamic window
   return L;
 }
 
-__host__ __device__ inline uint32_t pw_tmem_cols(const PwTc& p) {
+__host__ __device__ inline uint32_t pw_tmem_cols_dx(const PwTc& p) {
   if (p.zlen) return 2u * p.Np + (uint32_t)p.NA * (2u * (p.C1p + p.C2p) + 2u * p.Ks);   // T lives in the per-tile operand buffer
   return 2u * p.Np + 2u * p.Ks + 2u * (uint32_t)p.NA * (p.C1p + p.C2p);
 }
+// weight-gradient variant: its [MW x NW] accumulator follows, 32-column aligned
+__host__ __device__ inline uint32_t pw_tmem_wcol(const PwTc& p) { return (pw_tmem_cols_dx(p) + 31u) & ~31u; }
+template <bool WG>
+__host__ __device__ inline uint32_t pw_tmem_cols(const PwTc& p) { return WG ? pw_tmem_wcol(p) + p.NW : pw_tmem_cols_dx(p); }
 
 // MODE 1: no activation;  2: GELU;  3: multiply by GELU'(dz);  0: generic (runtime act / dact, add, mul)
 template <int MODE>
@@ -108,24 +123,27 @@ __device__ __forceinline__ float epi_value(float z, float mulv, float dzv, int a
   return v;
 }
 
-template <int MODE>
+// WG: also the 1x1 weight gradient of the dx pass (MODE 1 only; see PwTc::MW; tm2 is then the XW map, there is no second
+// 1x1 operand)
+template <int MODE, bool WG>
 __global__ void __launch_bounds__(kThreads, 1)
 k_pw_tc(const __grid_constant__ CUtensorMap tm1, const __grid_constant__ CUtensorMap tm2, const __grid_constant__ CUtensorMap tm3,
         const PwTc p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-  const PwLayout L = pw_layout(p);
+  const PwLayout L = pw_layout<WG>(p);
   uint64_t* full = (uint64_t*)(smem + L.bars);
   uint64_t* empty = full + p.S;
   uint64_t* a_full = empty + p.S;
   uint64_t* a_empty = a_full + 2;
   uint64_t* acc_full = a_empty + 2;
   uint64_t* acc_empty = acc_full + 2;
-  uint32_t* tslot = (uint32_t*)(acc_empty + 2);
+  uint64_t* wdone = acc_empty + 2;                       // WG only
+  uint32_t* tslot = (uint32_t*)(acc_empty + 2 + (WG ? 1 : 0));
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   uint32_t ncols = 32;
-  while (ncols < pw_tmem_cols(p)) ncols <<= 1;
+  while (ncols < pw_tmem_cols<WG>(p)) ncols <<= 1;
 
   // ---- one-time setup: weights (hi/lo, K-major core-matrix layout), bias, barriers, TMEM ----
   for (int i = tid; i < p.Np * p.C1p; i += kThreads) {
@@ -152,6 +170,19 @@ k_pw_tc(const __grid_constant__ CUtensorMap tm1, const __grid_constant__ CUtenso
     ((float*)(smem + L.tzh))[i] = hi;
     ((float*)(smem + L.tzl))[i] = tf32_rna(v - hi);
   }
+  if (WG) {
+    // the rows no TMA box writes: the lo copies start (and in single-pass mode stay) zero, the ones block of every XW box
+    // stays 1
+    for (uint32_t i = tid; i < (uint32_t)p.S * L.stage_bytes / 16u; i += kThreads)
+      *(float4*)(smem + L.stages + i * 16u) = make_float4(0.f, 0.f, 0.f, 0.f);
+    __syncthreads();
+    const uint32_t ones = (uint32_t)(p.NW - 2 * p.Cxp) * 8u;   // float4 per box
+    for (uint32_t i = tid; i < (uint32_t)p.S * 4u * ones; i += kThreads) {
+      const uint32_t s = i / (4u * ones), r = i - s * 4u * ones, j = r / ones;
+      *(float4*)(smem + L.stages + s * L.stage_bytes + L.xw + j * (uint32_t)p.NW * 128u + (uint32_t)p.Cxp * 256u + (r - j * ones) * 16u) =
+          make_float4(1.f, 1.f, 1.f, 1.f);
+    }
+  }
   if (tid == 0) {
     // a stage is free when its MMAs have completed and (dz ring) every epilogue thread has taken its dz values
     for (int s = 0; s < p.S; s++) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1 + ((MODE == 3 && p.Cz) ? kGroupThreadsPw : 0)); }
@@ -159,11 +190,12 @@ k_pw_tc(const __grid_constant__ CUtensorMap tm1, const __grid_constant__ CUtenso
       mbar_init(&a_full[a], 128); mbar_init(&a_empty[a], 1);
       mbar_init(&acc_full[a], 1); mbar_init(&acc_empty[a], kGroupThreadsPw);
     }
+    if (WG) mbar_init(wdone, 1);
     fence_barrier_init();
   }
   fence_proxy_async();
   if (warp == 1) tmem_alloc(tslot, ncols);
-  if (warp == 0 && lane == 0) { tma_prefetch_desc(&tm1); if (p.C2p) tma_prefetch_desc(&tm2); if (MODE == 3 && p.Cz) tma_prefetch_desc(&tm3); }
+  if (warp == 0 && lane == 0) { tma_prefetch_desc(&tm1); if (p.C2p || WG) tma_prefetch_desc(&tm2); if (MODE == 3 && p.Cz) tma_prefetch_desc(&tm3); }
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -172,6 +204,7 @@ k_pw_tc(const __grid_constant__ CUtensorMap tm1, const __grid_constant__ CUtenso
   const uint32_t x_width = 2u * (p.C1p + p.C2p);
   const uint32_t a_base = p.zlen ? tbase + 2u * p.Np : t_lo + p.Ks;
   const uint32_t a_width = p.zlen ? x_width + 2u * p.Ks : x_width;                    // 3-D: [X hi | lo ...][T hi | T lo] per buffer
+  const uint32_t t_w = tbase + pw_tmem_wcol(p);                                        // WG: the weight-gradient accumulator
 
   const uint32_t xb1 = (uint32_t)p.C1p * 512, xb2 = (uint32_t)p.C2p * 512, ab = (uint32_t)p.Ks * p.Np * 4;
   // each CTA owns a contiguous run of tiles (sequential DRAM pages per channel row, same sample for A')
@@ -181,7 +214,7 @@ k_pw_tc(const __grid_constant__ CUtensorMap tm1, const __grid_constant__ CUtenso
   if (warp == 0) {
     // ===================== TMA producer =====================
     if (lane == 0) {
-      const uint32_t bytes = xb1 + xb2 + ab + ((MODE == 3) ? (uint32_t)p.Cz * 512 : 0u);
+      const uint32_t bytes = xb1 + xb2 + ab + ((MODE == 3) ? (uint32_t)p.Cz * 512 : 0u) + (WG ? (uint32_t)p.Cxp * 512 : 0u);
       int it = 0;
       for (long tile = t_first; tile < t_end; tile++, it++) {
         const int s = it % p.S;
@@ -191,7 +224,14 @@ k_pw_tc(const __grid_constant__ CUtensorMap tm1, const __grid_constant__ CUtenso
         uint8_t* st = smem + L.stages + (size_t)s * L.stage_bytes;
         const int b = (int)(tile / p.tiles_per_img);
         const int t_in_img = (int)(tile - (long)b * p.tiles_per_img);
-        tma_load_3d(st, &tm1, &full[s], t_in_img * 128, 0, b);
+        if (WG) {
+          for (int j = 0; j < 4; j++) {
+            tma_load_3d(st + (uint32_t)j * p.C1p * 256u, &tm1, &full[s], t_in_img * 128 + 32 * j, 0, b);
+            tma_load_3d(st + L.xw + (uint32_t)j * p.NW * 128u, &tm2, &full[s], t_in_img * 128 + 32 * j, 0, b);
+          }
+        } else {
+          tma_load_3d(st, &tm1, &full[s], t_in_img * 128, 0, b);
+        }
         if (p.C2p) tma_load_3d(st + L.x2, &tm2, &full[s], t_in_img * 128, 0, b);
         if (MODE == 3 && p.Cz) tma_load_3d(st + L.dz, &tm3, &full[s], t_in_img * 128, 0, b);
         if (p.Ks) {
@@ -263,10 +303,32 @@ k_pw_tc(const __grid_constant__ CUtensorMap tm1, const __grid_constant__ CUtenso
           }
         }
         if (elect_one()) {
-          mma_commit(&empty[s]);
+          if (!WG) mma_commit(&empty[s]);
           mma_commit(&a_empty[xi]);
           mma_commit(&acc_full[a]);
         }
+        __syncwarp();
+        if (WG) {
+          // dWp += [X1 hi ; X1 lo] x [XW hi ; XW lo ; ones]^T over the tile's 128 px (K), both operands K-major SW128 boxes in
+          // the stage (the lo rows were written by the converter before it arrived on a_full); issued after the commits of
+          // the dx accumulator so that its epilogue does not wait for them
+          if (elect_one()) {
+            const uint32_t idesc_w = idesc_tf32(p.MW, p.NW, 0, 0);
+#pragma unroll 1
+            for (int j = 0; j < 4; j++) {
+              const uint64_t dg = smem_desc(st + (uint32_t)j * p.C1p * 256u, 16, 1024, LAYOUT_SW128);
+              const uint64_t dxw = smem_desc(st + L.xw + (uint32_t)j * p.NW * 128u, 16, 1024, LAYOUT_SW128);
+#pragma unroll
+              for (int ks = 0; ks < 4; ks++)
+                mma_tf32_ss(t_w, dg + (uint64_t)(ks * 2), dxw + (uint64_t)(ks * 2), idesc_w, (it > 0 || j > 0 || ks > 0) ? 1u : 0u);
+            }
+            mma_commit(&empty[s]);
+          }
+          __syncwarp();
+        }
+      }
+      if (WG) {
+        if (elect_one()) mma_commit(wdone);
         __syncwarp();
       }
     }
@@ -311,14 +373,47 @@ k_pw_tc(const __grid_constant__ CUtensorMap tm1, const __grid_constant__ CUtenso
       tc_fence_after();
       const uint32_t sx = smem_u32(smem) + L.stages + (uint32_t)s * L.stage_bytes + (uint32_t)m * 4u;
       const uint32_t xa = a_base + (uint32_t)a * a_width + lane_base;
-      for (int c0 = 0; c0 < p.C1p; c0 += 8) {
-        float hi[8], lo[8];
+      if (WG) {
+        // X1 from its SW128 box (pixel m: box m / 32, 16-byte chunk (m / 4) % 8 of row c swizzled by c % 8 -- a warp reads one
+        // 128-byte row per channel); the lo values also go to the rows after the box, the weight-gradient A operand
+        const uint32_t stg = smem_u32(smem) + L.stages + (uint32_t)s * L.stage_bytes;
+        const uint32_t gb = stg + (uint32_t)(m >> 5) * (uint32_t)p.C1p * 256u + (uint32_t)(m & 3) * 4u;
+        const uint32_t sw = (uint32_t)(m >> 2) & 7u;
+        const bool lo_rows = p.npass == 3;
+        for (int c0 = 0; c0 < p.C1p; c0 += 8) {
+          float hi[8], lo[8];
 #pragma unroll
-        for (int j = 0; j < 8; j++) hi[j] = lds_f32(sx + (uint32_t)(c0 + j) * 512u);
+          for (int j = 0; j < 8; j++) hi[j] = lds_f32(gb + (uint32_t)(c0 + j) * 128u + ((sw ^ (uint32_t)j) << 4));
 #pragma unroll
-        for (int j = 0; j < 8; j++) lo[j] = tf32_lo(hi[j]);
-        tmem_st8(xa + c0, hi);
-        tmem_st8(xa + p.C1p + c0, lo);
+          for (int j = 0; j < 8; j++) lo[j] = tf32_lo(hi[j]);
+          tmem_st8(xa + c0, hi);
+          tmem_st8(xa + p.C1p + c0, lo);
+          if (lo_rows) {
+#pragma unroll
+            for (int j = 0; j < 8; j++) sts_f32(gb + (uint32_t)(p.C1p + c0 + j) * 128u + ((sw ^ (uint32_t)j) << 4), lo[j]);
+          }
+        }
+        if (lo_rows) {
+          // XW lo rows: elementwise copy of each box (same swizzle phase: Cxp is a multiple of 8 rows)
+          const uint32_t per_box = (uint32_t)p.Cxp * 8u;   // float4 per box
+          for (int j = 0; j < 4; j++) {
+            const uint32_t xb = stg + L.xw + (uint32_t)j * (uint32_t)p.NW * 128u;
+            for (uint32_t i = (uint32_t)m; i < per_box; i += 128u) {
+              const float4 v = lds_v4(xb + i * 16u);
+              sts_v4(xb + (uint32_t)p.Cxp * 128u + i * 16u, make_float4(tf32_lo(v.x), tf32_lo(v.y), tf32_lo(v.z), tf32_lo(v.w)));
+            }
+          }
+        }
+      } else {
+        for (int c0 = 0; c0 < p.C1p; c0 += 8) {
+          float hi[8], lo[8];
+#pragma unroll
+          for (int j = 0; j < 8; j++) hi[j] = lds_f32(sx + (uint32_t)(c0 + j) * 512u);
+#pragma unroll
+          for (int j = 0; j < 8; j++) lo[j] = tf32_lo(hi[j]);
+          tmem_st8(xa + c0, hi);
+          tmem_st8(xa + p.C1p + c0, lo);
+        }
       }
       if (p.C2p) {
         const uint32_t sx2 = sx + L.x2;
@@ -356,7 +451,37 @@ k_pw_tc(const __grid_constant__ CUtensorMap tm1, const __grid_constant__ CUtenso
       }
       tmem_st_wait();
       tc_fence_before();
+      if (WG) fence_proxy_async();
       mbar_arrive(&a_full[a]);
+    }
+    if (WG) {
+      // read-out of the weight gradient: accumulator row r = X1 hi row r (r < C1p) or lo row r - C1p; columns [0, Cxp) +
+      // [Cxp, 2 Cxp) are the XW hi and lo products, column 2 Cxp the ones (db).  The hi rows write the CTA's partial in the
+      // first gridDim.x slots, the lo rows theirs in the next gridDim.x; the reduction adds both in a fixed order.
+      // (M = 64: row r lives in TMEM lane 32 (r / 16) + r % 16.)
+      mbar_wait(wdone, 0);
+      tc_fence_after();
+      const int r = p.MW == 64 ? quad * 16 + (lane & 15) : m;
+      const int half = r >= p.C1p ? 1 : 0, o = r - half * p.C1p;
+      const bool own = (p.MW != 64 || lane < 16) && o < p.C1;
+      const bool any = t_end > t_first;
+      float* pout = p.wpart + ((size_t)half * gridDim.x + blockIdx.x) * ((size_t)p.C1 * p.Cx + p.C1);
+      const uint32_t tw = t_w + lane_base;
+      for (int c0 = 0; c0 < p.Cxp; c0 += 8) {
+        float v[8], u[8];
+        tmem_ld8(tw + (uint32_t)c0, v);
+        tmem_ld8(tw + (uint32_t)(p.Cxp + c0), u);
+        tmem_ld_wait();
+        if (own) {
+#pragma unroll
+          for (int j = 0; j < 8; j++)
+            if (c0 + j < p.Cx) pout[(size_t)o * p.Cx + c0 + j] = any ? v[j] + u[j] : 0.f;
+        }
+      }
+      float v[8];
+      tmem_ld8(tw + 2u * (uint32_t)p.Cxp, v);
+      tmem_ld_wait();
+      if (own) pout[(size_t)p.C1 * p.Cx + o] = any ? v[0] : 0.f;
     }
   } else {
     // ===================== epilogue: 8 warps per tile = 4 lane quadrants x 2 column parts, two groups =====================
@@ -624,9 +749,10 @@ extern "C" int b2no_set_tensor_core_mode(int on) {
 }
 
 // Returns 0 when the tile kernel ran, 1 when the shape is not eligible (caller falls back to the CUDA-core
-// kernel), otherwise an error code.
+// kernel), otherwise an error code.  With `wg` only the weight-gradient variant is eligible, and nothing is launched when it
+// is not.
 int b2no_tc_pointwise(const b2no_plan* plan, int which, const float* spec, float* y, float* work, int batch, int channels,
-                      long pixels, const b2no_epilogue* e, cudaStream_t st) {
+                      long pixels, const b2no_epilogue* e, cudaStream_t st, const b2no_tc_wg* wg) {
   if (!b2no_tc_available()) return 1;
   if (!e || !e->pw_w || !e->pw_x || e->pw_ci < 1) return 1;          // needs at least one 1x1 operand (the TMA-fed A tile)
   if (pixels % 128 != 0 || channels > 256 || e->pw_ci > 128 || e->pw2_ci > 128) return 1;
@@ -673,14 +799,29 @@ int b2no_tc_pointwise(const b2no_plan* plan, int which, const float* spec, float
     p.ahi = work;
     p.alo = work;
   }
+  if (wg) {
+    // 2-D plans, one 1x1 operand of <= 64 channels ([hi ; lo] rows fill at most M = 128), XW of <= 112 channels (N <= 256)
+    if (!spec || three_d || has2 || p.C1p > 64 || wg->ci < 1 || wg->ci > 112 || ((uintptr_t)wg->x & 15)) return 1;
+    p.Cx = wg->ci; p.Cxp = b2no_round_up(wg->ci, 8);
+    p.MW = 2 * p.C1p <= 64 ? 64 : 128;
+    p.NW = b2no_round_up(2 * p.Cxp + 1, p.MW == 64 ? 8 : 16);   // the ones block: 8 or 16 rows
+    p.wpart = wg->partial;
+  }
   p.NA = 2;
-  if (pw_tmem_cols(p) > 512) p.NA = 1;          // wide operands: one A buffer (the converter then waits for the tile's MMAs)
-  if (pw_tmem_cols(p) > 512) return 1;
+  auto tmem_cols = [&]() { return wg ? pw_tmem_cols<true>(p) : pw_tmem_cols<false>(p); };
+  auto layout = [&]() { return wg ? pw_layout<true>(p) : pw_layout<false>(p); };
+  if (tmem_cols() > 512) p.NA = 1;              // wide operands: one A buffer (the converter then waits for the tile's MMAs)
+  if (tmem_cols() > 512) return 1;
   const bool extras = p.add || p.mul || p.gate_z;
   int mode = 0;
   if (!extras && !p.dact && p.act == B2NO_ACT_NONE && !p.preact) mode = 1;
   else if (!extras && !p.dact && p.act == B2NO_ACT_GELU) mode = 2;
   else if (!extras && p.dact == B2NO_ACT_GELU && p.act == B2NO_ACT_NONE && !p.preact) mode = 3;
+  // The dx pass without activation only.  Measured on a B200 (1000 W) at the cfg2 layer shape (B 64, 32 ch, 128^2, modes 12,
+  // inputs larger than L2, scripts/fused_wgrad_timing.py): this variant 172 us against 179 us for k_pw_tc<1> + k_wgrad_tc +
+  // reduce; with GELU'(dz) (MODE 3) 203 us against 193 us -- the dz tile makes a stage 90 KB, two fit next to the weights
+  // (102 KB of payload in flight against six stages of k_pw_tc<3> alone), so MODE 3 keeps the two launches.
+  if (wg && mode != 1) return 1;
   // dz through the TMA ring: enabled for the single-pass case (Co <= 32: every epilogue thread takes its 8 values and
   // releases the stage at once), which is what the parity tests and the bench exercise; wider layers keep the per-thread
   // loads until the multi-pass variant of the ring has its own GPU test
@@ -691,13 +832,13 @@ int b2no_tc_pointwise(const b2no_plan* plan, int which, const float* spec, float
   B2NO_CHECK_CUDA(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
   PwLayout L;
   for (p.S = 6; p.S >= 2; p.S--) {
-    L = pw_layout(p);
+    L = layout();
     if ((int)L.total <= max_smem) break;
   }
   if (p.S < 3 && p.Cz) {          // not enough room for a useful ring with the dz tile: plain loads instead
     p.Cz = 0;
     for (p.S = 6; p.S >= 2; p.S--) {
-      L = pw_layout(p);
+      L = layout();
       if ((int)L.total <= max_smem) break;
     }
   }
@@ -708,8 +849,15 @@ int b2no_tc_pointwise(const b2no_plan* plan, int which, const float* spec, float
     uint64_t dims[3] = {(uint64_t)pixels, (uint64_t)p.C1, (uint64_t)batch};
     uint64_t str[3] = {4, (uint64_t)pixels * 4, (uint64_t)pixels * 4 * p.C1};
     uint32_t box[3] = {128, (uint32_t)p.C1p, 1};
-    if (make_tmap_f32(&tm1, e->pw_x, 3, dims, str, box, CU_TENSOR_MAP_SWIZZLE_NONE)) return 1;
+    if (wg) box[0] = 32;                         // [32 px x C1p] boxes with the 128-byte swizzle: K-major operands
+    if (make_tmap_f32(&tm1, e->pw_x, 3, dims, str, box, wg ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE)) return 1;
     tm2 = tm1;
+    if (wg) {
+      uint64_t dimsw[3] = {(uint64_t)pixels, (uint64_t)p.Cx, (uint64_t)batch};
+      uint64_t strw[3] = {4, (uint64_t)pixels * 4, (uint64_t)pixels * 4 * p.Cx};
+      uint32_t boxw[3] = {32, (uint32_t)p.Cxp, 1};
+      if (make_tmap_f32(&tm2, wg->x, 3, dimsw, strw, boxw, CU_TENSOR_MAP_SWIZZLE_128B)) return 1;
+    }
     if (has2) {
       uint64_t dims2[3] = {(uint64_t)pixels, (uint64_t)p.C2, (uint64_t)batch};
       uint64_t str2[3] = {4, (uint64_t)pixels * 4, (uint64_t)pixels * 4 * p.C2};
@@ -765,16 +913,21 @@ int b2no_tc_pointwise(const b2no_plan* plan, int which, const float* spec, float
   p.tiles_per_cta = (p.tiles + grid - 1) / grid;
   grid = (p.tiles + p.tiles_per_cta - 1) / p.tiles_per_cta;
   p.npass = b2no_tc_passes();
-#define LAUNCH(M)                                                                                                  \
-  do {                                                                                                             \
-    B2NO_CHECK_CUDA(cudaFuncSetAttribute(k_pw_tc<M>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total));  \
-    k_pw_tc<M><<<(unsigned)grid, kThreads, L.total, st>>>(tm1, tm2, tm3, p);                                           \
+#define LAUNCH(M, W)                                                                                                  \
+  do {                                                                                                                \
+    B2NO_CHECK_CUDA(cudaFuncSetAttribute(k_pw_tc<M, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total));  \
+    k_pw_tc<M, W><<<(unsigned)grid, kThreads, L.total, st>>>(tm1, tm2, tm3, p);                                           \
   } while (0)
-  switch (mode) {
-    case 1: LAUNCH(1); break;
-    case 2: LAUNCH(2); break;
-    case 3: LAUNCH(3); break;
-    default: LAUNCH(0); break;
+  if (wg) {
+    LAUNCH(1, true);
+    *wg->nblk = 2 * (int)grid;                    // the hi-row and lo-row partials of every CTA
+  } else {
+    switch (mode) {
+      case 1: LAUNCH(1, false); break;
+      case 2: LAUNCH(2, false); break;
+      case 3: LAUNCH(3, false); break;
+      default: LAUNCH(0, false); break;
+    }
   }
 #undef LAUNCH
   B2NO_LAUNCH_CHECK();

@@ -21,6 +21,12 @@ def _contig(t: torch.Tensor) -> torch.Tensor:
     return t if t.is_contiguous() else t.contiguous()
 
 
+def _fused_wgrad_ok(g: torch.Tensor) -> bool:
+    """The dx pass may also compute the 1x1 weight gradient (ops.dft_inverse_wgrad, which itself declines shapes it does
+    not support): CUDA tensors only."""
+    return g.is_cuda
+
+
 def _geom_has_overlap(geom: SpecGeom) -> bool:
     g = geom.resolved()
     return any(2 * g.half[j] > g.nfft[j] for j in range(g.ndim - 1))
@@ -77,8 +83,15 @@ class SpectralBlockFn(torch.autograd.Function):
         dcorners: List[Optional[torch.Tensor]] = [None] * len(det)
         if need_w:
             dcorners = ops.mix_dw(plan, xh, gyh, det, needs_zero=_geom_has_overlap(geom))
+        fused = None
+        if need_x:
+            gxh = ops.mix(plan, 1, gyh, det, ci, co)
+            epi = ops.make_epilogue(pw_w=pw2d, pw_x=gz if pw2d is not None else None, pw_transposed=True)
+            if need_pw and _fused_wgrad_ok(gz):
+                fused = ops.dft_inverse_wgrad(plan, 1, gxh, epi, x, need_bias=need_b)
+            dx = fused[0] if fused is not None else ops.dft_inverse(plan, 1, gxh, epi)
         if need_pw:
-            dpw, db2 = ops.pw_wgrad(gz, x, need_bias=need_b)
+            dpw, db2 = fused[1:] if fused is not None else ops.pw_wgrad(gz, x, need_bias=need_b)
             dpw = dpw.reshape(ctx.pw_shape)
             if need_b:
                 dbias = db2.reshape(ctx.bias_shape)
@@ -86,10 +99,6 @@ class SpectralBlockFn(torch.autograd.Function):
             # dbias[o] = sum_{b,n} gz = DC mode of the (scaled) truncated DFT: gYh[b,o,0..0] = s_i * sum_n gz
             dc = gyh.reshape(B, co, -1)[:, :, 0].real.sum(dim=0) / plan.s_i
             dbias = dc.reshape(ctx.bias_shape)
-        if need_x:
-            gxh = ops.mix(plan, 1, gyh, det, ci, co)
-            epi = ops.make_epilogue(pw_w=pw2d, pw_x=gz if pw2d is not None else None, pw_transposed=True)
-            dx = ops.dft_inverse(plan, 1, gxh, epi)
         return (dx, dbias, dpw, None, None) + tuple(dcorners)
 
 
@@ -164,15 +173,28 @@ class FNOStackFn(torch.autograd.Function):
                 dcs = ops.mix_dw(plan, xh, gyh, det, needs_zero=_geom_has_overlap(geom))
                 for j in range(nc):
                     grads[l * per + 1 + j] = dcs[j]
-            if need_bias or need[0]:
-                dpw, _ = ops.pw_wgrad(g, x, need_bias=need_bias, db_out=dbias[l] if need_bias else None)
-                grads[l * per] = dpw.reshape(pw_shape)
+            need_wgrad = need_bias or need[0]
+            db_out = dbias[l] if need_bias else None
+            fused = None
             if l > 0 or ctx.needs_input_grad[0]:
                 gxh = ops.mix(plan, 1, gyh, det, ci, co)
                 zprev = saved[(l - 1) * per_s + 2] if (l > 0 and meta[l - 1][3]) else None
                 epi = ops.make_epilogue(pw_w=pw2d, pw_x=g, pw_transposed=True, dact_z=zprev,
                                         dact=acts[l - 1] if zprev is not None else None)
-                g = ops.dft_inverse(plan, 1, gxh, epi)
+                # the dx pass reads g tile by tile anyway: it also computes dWp and dbias[l] when it can
+                if need_wgrad and _fused_wgrad_ok(g):
+                    fused = ops.dft_inverse_wgrad(plan, 1, gxh, epi, x, need_bias=need_bias, db_out=db_out)
+                if fused is None:
+                    if need_wgrad:
+                        dpw, _ = ops.pw_wgrad(g, x, need_bias=need_bias, db_out=db_out)
+                        grads[l * per] = dpw.reshape(pw_shape)
+                    g = ops.dft_inverse(plan, 1, gxh, epi)
+                else:
+                    g = fused[0]
+                    grads[l * per] = fused[1].reshape(pw_shape)
+            elif need_wgrad:
+                dpw, _ = ops.pw_wgrad(g, x, need_bias=need_bias, db_out=db_out)
+                grads[l * per] = dpw.reshape(pw_shape)
         return (g if ctx.needs_input_grad[0] else None, None, None, None,
                 dbias.reshape(ctx.bias_shape) if need_bias else None) + tuple(grads)
 

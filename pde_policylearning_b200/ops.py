@@ -342,6 +342,36 @@ def pw_wgrad(g: torch.Tensor, x: torch.Tensor, need_bias: bool, db_out: Optional
     return dw, db
 
 
+def dft_inverse_wgrad(plan: Plan, which: int, spec: torch.Tensor, epi: Epilogue, x: torch.Tensor, need_bias: bool,
+                      db_out: Optional[torch.Tensor] = None):
+    """dft_inverse(plan, which, spec, epi) and pw_wgrad(g, x) in one pass over the pixel tiles, g = the epilogue's pw_x
+    (b2no_dft_inverse_wgrad).  Returns (y, dW (Co, Ci), db | None), or None -- with nothing computed -- when the fused pass
+    does not support the shape; the caller then makes the two calls."""
+    _require_cuda(spec, x)
+    assert spec.dtype == torch.complex64 and spec.is_contiguous()
+    assert x.dtype == torch.float32 and x.is_contiguous()
+    B, Cc = plan.spec_bc(spec)
+    grid = plan.geom.nout if which == 0 else plan.geom.nin
+    if tuple(x.shape) != (B, x.shape[1]) + tuple(grid):
+        raise ValueError(f"x {tuple(x.shape)} does not match batch {B} and grid {tuple(grid)}")
+    co, ci = int(epi.pw_ci), int(x.shape[1])
+    L = _lib.lib()
+    y = torch.empty((B, Cc) + tuple(grid), dtype=torch.float32, device=spec.device)
+    work = plan.workspace(B, Cc)
+    partial = torch.empty(int(L.b2no_pw_wgrad_scratch_floats(ci, co)), dtype=torch.float32, device=spec.device)
+    dw = torch.empty((co, ci), dtype=torch.float32, device=spec.device)
+    db = None
+    if need_bias:
+        db = db_out if db_out is not None else torch.empty((co,), dtype=torch.float32, device=spec.device)
+        assert db.is_contiguous() and db.numel() == co and db.dtype == torch.float32
+    rc = L.b2no_dft_inverse_wgrad(plan.handle, which, _ptr(spec), _ptr(y), _ptr(work), B, Cc, math.prod(grid), C.byref(epi),
+                                  _ptr(x), ci, _ptr(dw), _ptr(db), _ptr(partial), _stream())
+    if rc == -2:
+        return None
+    check(rc, "dft_inverse_wgrad")
+    return y, dw, db
+
+
 def mlp_head_fwd(x, w1, b1, w2, b2, act="gelu") -> torch.Tensor:
     B, ci = x.shape[:2]
     grid = tuple(x.shape[2:])
