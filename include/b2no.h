@@ -195,6 +195,26 @@ int b2no_mlp_head_bwd_fused_supported(int ci, int hidden, int64_t pixels);
 int b2no_mlp_head_bwd_fused(const float* x, const float* w1, const float* b1, const float* w2, const float* g, float* gx,
                             float* grads, float* partial, int batch, int ci, int hidden, int64_t pixels, int act,
                             const float* dact_z, int dact, void* stream);
+/* Fused head with out_channels = O = 2..4 (pinobserver.py:230-232 via PlanePredHead, :257-273, whose tail emits
+ * plane_num * out_dim channels; tfno.py:34-38 Projection with out_channels > 1):
+ *   out[b,o,p] = b2[o] + sum_j w2[o,j] * act( b1[(b),j] + sum_i w1[j,i] x[b,i,p] )
+ * w2 is (O, hidden) row-major, b2 (O) or NULL, out (batch, O, pixels); the hidden tensor is never written.  Tensor cores
+ * only: returns B2NO_E_UNSUPPORTED, having written nothing, when O is outside 2..4, pixels % 128 != 0, ci > 64,
+ * hidden > 512, x is not 16-byte aligned, the device has no tensor-core kernels or shared / tensor memory is too small. */
+int b2no_mlp_head_fwd_multi(const float* x, const float* w1, const float* b1, const float* w2, const float* b2, float* out,
+                            int batch, int ci, int hidden, int out_channels, int64_t pixels, int b1_per_sample, int act,
+                            void* stream);
+/* Input-gradient half of its backward, the O-output form of b2no_mlp_head_bwd (same reference lines):
+ *   f[b,j,p] = act'(z1[b,j,p]) sum_o g[b,o,p] w2[o,j];  gx[b,i,p] = sum_j w1[j,i] f[b,j,p] (* dact'(dact_z) when given);
+ *   dw2[o,j] = sum_{b,p} g[b,o,p] act(z1[b,j,p]) ((O, hidden));  gz (optional, (batch, hidden, pixels)) receives f for
+ *   b2no_pw_wgrad (dW1, db1).  g is (batch, O, pixels).  partial: b2no_mlp_head_bwd_multi_scratch_floats(hidden, O) floats.
+ * Returns B2NO_E_UNSUPPORTED, having written nothing, where b2no_mlp_head_bwd_multi_supported is 0 (same limits as the
+ * forward, and the shared-memory budget of the backward: e.g. ci = 64 with hidden = 256 does not fit). */
+int b2no_mlp_head_bwd_multi_supported(int ci, int hidden, int out_channels, int64_t pixels);
+int64_t b2no_mlp_head_bwd_multi_scratch_floats(int hidden, int out_channels);
+int b2no_mlp_head_bwd_multi(const float* x, const float* w1, const float* b1, const float* w2, const float* g, float* gx,
+                            float* gz, float* dw2, float* partial, int batch, int ci, int hidden, int out_channels,
+                            int64_t pixels, int b1_per_sample, int act, const float* dact_z, int dact, void* stream);
 /* RNO gate (rno.py:259): h_next = (1 - z) * h + z2 * hhat, and its backward */
 int b2no_rno_gate_fwd(const float* z, const float* z2, const float* hhat, const float* h, float* out,
                       int64_t n, void* stream);

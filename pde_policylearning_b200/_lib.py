@@ -118,6 +118,11 @@ def lib():
     L.b2no_mlp_head_bwd_fused_scratch_floats.restype = i64
     L.b2no_mlp_head_bwd_fused_scratch_floats.argtypes = [i32, i32]
     L.b2no_mlp_head_bwd_fused.argtypes = [vp] * 8 + [i32, i32, i32, i64, i32, vp, i32, vp]
+    L.b2no_mlp_head_fwd_multi.argtypes = [vp] * 6 + [i32, i32, i32, i32, i64, i32, i32, vp]
+    L.b2no_mlp_head_bwd_multi_supported.argtypes = [i32, i32, i32, i64]
+    L.b2no_mlp_head_bwd_multi_scratch_floats.restype = i64
+    L.b2no_mlp_head_bwd_multi_scratch_floats.argtypes = [i32, i32]
+    L.b2no_mlp_head_bwd_multi.argtypes = [vp] * 9 + [i32, i32, i32, i32, i64, i32, i32, vp, i32, vp]
     L.b2no_rno_gate_fwd.argtypes = [vp, vp, vp, vp, vp, i64, vp]
     L.b2no_rno_gate_bwd.argtypes = [vp] * 9 + [i64, vp]
     L.b2no_rno_cell_bwd.argtypes = [vp] * 7 + [i32, i32, i64, vp]
@@ -147,6 +152,8 @@ EXPORTS = [
     "b2no_dft_forward", "b2no_dft_inverse", "b2no_mix", "b2no_mix_dw",
     "b2no_act_bwd", "b2no_pw_wgrad_scratch_floats", "b2no_pw_wgrad", "b2no_dft_inverse_wgrad", "b2no_mlp_head_fwd", "b2no_mlp_head_bwd_scratch_floats", "b2no_mlp_head_bwd_supported", "b2no_mlp_head_bwd",
     "b2no_mlp_head_bwd_fused_scratch_floats", "b2no_mlp_head_bwd_fused_supported", "b2no_mlp_head_bwd_fused",
+    "b2no_mlp_head_fwd_multi", "b2no_mlp_head_bwd_multi_supported", "b2no_mlp_head_bwd_multi_scratch_floats",
+    "b2no_mlp_head_bwd_multi",
     "b2no_rno_gate_fwd", "b2no_rno_gate_bwd", "b2no_rno_cell_bwd", "b2no_rno_reset_bwd", "b2no_rel_l2_sums", "b2no_rel_l2_bwd",
     "b2no_rel_l2_finish", "b2no_rel_l2_bwd_g", "b2no_adam_step", "b2no_gather_segments",
     "b2no_tc_peak_probe", "b2no_pino_residual_scratch_floats", "b2no_pino_residual_fwd", "b2no_pino_residual_bwd",

@@ -43,15 +43,16 @@ struct MlpTc {
 
 struct MlpLayout { uint32_t w1h, w1l, w2h, w2l, b1, w2v, dw2, part, stages, stage_bytes, bars, total; };
 
-__host__ __device__ inline MlpLayout mlp_layout(const MlpTc& p) {
+// no: output channels of a backward launch (the w2 rows and dw2 accumulators kept in shared memory); 1 otherwise
+__host__ __device__ inline MlpLayout mlp_layout(const MlpTc& p, int no = 1) {
   MlpLayout L;
   uint32_t o = 0;
   const uint32_t wb1 = (uint32_t)p.Hp * p.Cip * 4, wb2 = (uint32_t)p.N2 * p.Hp * 4;
   L.w1h = o; o += wb1; L.w1l = o; o += wb1;
   L.w2h = o; o += wb2; L.w2l = o; o += wb2;
   L.b1 = o; o += (uint32_t)p.Hp * 4;
-  L.w2v = o; o += (uint32_t)p.Hp * 4;
-  L.dw2 = o; o += (uint32_t)p.Hp * 4;
+  L.w2v = o; o += (uint32_t)no * p.Hp * 4;
+  L.dw2 = o; o += (uint32_t)no * p.Hp * 4;
   L.part = o; o += 2 * 4 * 128 * 4;
   o = (o + 1023u) & ~1023u;
   L.stages = o;
@@ -68,12 +69,43 @@ __host__ __device__ inline uint32_t mlp_tmem_cols(const MlpTc& p) {
   return 2u * p.Cip + 128u + 128u * p.fbufs + 2u * p.N2;
 }
 
-template <bool GELU, bool BWD, bool DIRECT>
+// dw2[col] += sum over the warp's 32 pixels of ga[col] (kEW columns per lane): transposing butterfly; while a lane still
+// holds more than one column the halves are exchanged, afterwards plain xor-sums.  Returns the sum of column
+// lane >> (5 - log2 kEW), identical in the 32 / kEW lanes of each group.
+__device__ __forceinline__ float warp_column_sum(float (&ga)[kEW], int lane) {
+  int cnt = kEW;
+#pragma unroll
+  for (int s = 0; s < 5; s++) {
+    const int off = 16 >> s;
+    if (cnt > 1) {
+      const int hw = cnt >> 1;
+      const bool upper = (lane & off) != 0;
+#pragma unroll
+      for (int i = 0; i < kEW / 2; i++) {
+        if (i < hw) {
+          const float a0 = ga[i], a1 = ga[i + hw];
+          const float send = upper ? a0 : a1;
+          const float keep = upper ? a1 : a0;
+          ga[i] = keep + __shfl_xor_sync(0xffffffffu, send, off);
+        }
+      }
+      cnt = hw;
+    } else {
+      ga[0] += __shfl_xor_sync(0xffffffffu, ga[0], off);
+    }
+  }
+  return ga[0];
+}
+
+// NO: output channels of the head (backward only; the forward takes p.Co2 at run time).  With NO > 1 the backward reads NO
+// upstream gradients per pixel, forms f[j] = act'(z1[j]) sum_o g[o] w2[o,j] and keeps NO dw2 rows.
+template <bool GELU, bool BWD, bool DIRECT, int NO = 1>
 __global__ void __launch_bounds__(kThreadsMlp, 1)
 k_mlp_tc(const __grid_constant__ CUtensorMap tmx, const MlpTc p) {
+  static_assert(NO >= 1 && (NO == 1 || (BWD && !DIRECT)), "several outputs: backward kernel only");
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-  const MlpLayout L = mlp_layout(p);
+  const MlpLayout L = mlp_layout(p, NO);
   uint64_t* full = (uint64_t*)(smem + L.bars);
   uint64_t* empty = full + p.S;
   uint64_t* x_full = empty + p.S;
@@ -114,8 +146,11 @@ k_mlp_tc(const __grid_constant__ CUtensorMap tmx, const MlpTc p) {
   }
   for (int i = tid; i < p.Hp; i += kThreadsMlp) {
     ((float*)(smem + L.b1))[i] = (!p.b1_per_sample && p.b1 && i < p.H) ? p.b1[i] : 0.f;
-    ((float*)(smem + L.w2v))[i] = ((bwd || direct) && i < p.H) ? p.w2[i] : 0.f;
-    ((float*)(smem + L.dw2))[i] = 0.f;
+#pragma unroll
+    for (int o = 0; o < NO; o++) {
+      ((float*)(smem + L.w2v))[o * p.Hp + i] = ((bwd || direct) && i < p.H) ? p.w2[(size_t)o * p.H + i] : 0.f;
+      ((float*)(smem + L.dw2))[o * p.Hp + i] = 0.f;
+    }
   }
   if (tid == 0) {
     for (int s = 0; s < p.S; s++) { mbar_init(&full[s], 1); mbar_init(&empty[s], 128); }
@@ -337,7 +372,10 @@ k_mlp_tc(const __grid_constant__ CUtensorMap tmx, const MlpTc p) {
     for (long tile = t_first; tile < t_end; tile++, it++) {
       const int b = (int)(tile / p.tiles_per_img);
       const long px = (tile - (long)b * p.tiles_per_img) * 128 + t;
-      const float gv = bwd ? __ldg(p.g + (size_t)b * p.P + px) : 0.f;
+      float gvo[NO];
+#pragma unroll
+      for (int o = 0; o < NO; o++) gvo[o] = bwd ? __ldg(p.g + ((size_t)b * NO + o) * p.P + px) : 0.f;
+      const float gv = gvo[0];
       const float* b1g = p.b1_per_sample ? p.b1 + (size_t)b * p.H : nullptr;
       float2 oacc = make_float2(0.f, 0.f);
       for (int c = 0; c < NC; c++) {
@@ -366,7 +404,21 @@ k_mlp_tc(const __grid_constant__ CUtensorMap tmx, const MlpTc p) {
           // packed fp32x2 math: one FMA-pipe instruction per two hidden units
           float2* v2 = reinterpret_cast<float2*>(v);
           const float2* b2 = reinterpret_cast<const float2*>(bj);
-          if (bwd) {
+          if (bwd && NO > 1) {
+            // ga = gelu(z) (scaled by each g[o] in the dw2 reduction below), f = gelu'(z) sum_o g[o] w2[o,j]
+            float2* ga2 = reinterpret_cast<float2*>(ga);
+#pragma unroll
+            for (int j = 0; j < kEW / 2; j++) {
+              float2 val, grad;
+              b2no_gelu2_both(__fadd2_rn(v2[j], b2[j]), &val, &grad);
+              float2 s = __fmul2_rn(b2no_f2(gvo[0]), *reinterpret_cast<const float2*>(sw2 + col0 + 2 * j));
+#pragma unroll
+              for (int o = 1; o < NO; o++)
+                s = __ffma2_rn(b2no_f2(gvo[o]), *reinterpret_cast<const float2*>(sw2 + o * p.Hp + col0 + 2 * j), s);
+              ga2[j] = val;
+              v2[j] = __fmul2_rn(s, grad);
+            }
+          } else if (bwd) {
             float2* ga2 = reinterpret_cast<float2*>(ga);
             const float2 gv2 = b2no_f2(gv);
 #pragma unroll
@@ -391,7 +443,13 @@ k_mlp_tc(const __grid_constant__ CUtensorMap tmx, const MlpTc p) {
 #pragma unroll
           for (int j = 0; j < kEW; j++) {
             const float z = v[j] + bj[j];
-            if (bwd) {
+            if (bwd && NO > 1) {
+              float s = gvo[0] * sw2[col0 + j];
+#pragma unroll
+              for (int o = 1; o < NO; o++) s = fmaf(gvo[o], sw2[o * p.Hp + col0 + j], s);
+              ga[j] = b2no_act(z, p.act);
+              v[j] = s * b2no_act_grad(z, p.act);
+            } else if (bwd) {
               ga[j] = gv * b2no_act(z, p.act);
               v[j] = gv * sw2[col0 + j] * b2no_act_grad(z, p.act);
             } else if (direct) {
@@ -409,33 +467,21 @@ k_mlp_tc(const __grid_constant__ CUtensorMap tmx, const MlpTc p) {
             for (int j = 0; j < kEW; j++)
               if (col0 + j < p.H) gp[(size_t)j * p.P] = v[j];
           }
-          // dw2[col] += sum over the warp's 32 pixels of g * act(z): transposing butterfly; while a lane still holds
-          // more than one column the halves are exchanged, afterwards plain xor-sums.  Column kept by lane l:
-          // l >> (5 - log2 kEW); one lane of each group of 32 / kEW adds it to the shared-memory total.
-          {
-            int cnt = kEW;
+          // dw2[o,col] += sum over the warp's 32 pixels of g[o] * act(z) (warp_column_sum); one lane of each group of
+          // 32 / kEW adds it to the shared-memory total
+          constexpr int kDup = 32 / kEW;
+          if (NO == 1) {
+            const float s = warp_column_sum(ga, lane);
+            if ((lane & (kDup - 1)) == 0) atomicAdd(&sdw2[col0 + lane / kDup], s);
+          } else {
 #pragma unroll
-            for (int s = 0; s < 5; s++) {
-              const int off = 16 >> s;
-              if (cnt > 1) {
-                const int hw = cnt >> 1;
-                const bool upper = (lane & off) != 0;
+            for (int o = 0; o < NO; o++) {
+              float go[kEW];
 #pragma unroll
-                for (int i = 0; i < kEW / 2; i++) {
-                  if (i < hw) {
-                    const float a0 = ga[i], a1 = ga[i + hw];
-                    const float send = upper ? a0 : a1;
-                    const float keep = upper ? a1 : a0;
-                    ga[i] = keep + __shfl_xor_sync(0xffffffffu, send, off);
-                  }
-                }
-                cnt = hw;
-              } else {
-                ga[0] += __shfl_xor_sync(0xffffffffu, ga[0], off);
-              }
+              for (int j = 0; j < kEW; j++) go[j] = gvo[o] * ga[j];
+              const float s = warp_column_sum(go, lane);
+              if ((lane & (kDup - 1)) == 0) atomicAdd(&sdw2[o * p.Hp + col0 + lane / kDup], s);
             }
-            constexpr int kDup = 32 / kEW;
-            if ((lane & (kDup - 1)) == 0) atomicAdd(&sdw2[col0 + lane / kDup], ga[0]);
           }
         }
         const int fb = (int)(n % p.fbufs);
@@ -498,7 +544,10 @@ k_mlp_tc(const __grid_constant__ CUtensorMap tmx, const MlpTc p) {
   tc_fence_before();
   __syncthreads();
   if (bwd && p.dw2_partial)
-    for (int i = tid; i < p.H; i += kThreadsMlp) p.dw2_partial[(size_t)blockIdx.x * p.H + i] = ((float*)(smem + L.dw2))[i];
+    for (int i = tid; i < p.H; i += kThreadsMlp)
+#pragma unroll
+      for (int o = 0; o < NO; o++)
+        p.dw2_partial[((size_t)blockIdx.x * NO + o) * p.H + i] = ((float*)(smem + L.dw2))[o * p.Hp + i];
   if (warp == 1) tmem_dealloc(tbase, ncols);
 }
 
@@ -530,6 +579,8 @@ k_sum_partials(const float* __restrict__ partial, float* __restrict__ out, int n
 int mlp_launch(MlpTc& p, const float* x, int batch, long pixels, cudaStream_t st, int* grid_out) {
   if (!b2no_tc_available()) return 1;
   if (pixels % 128 != 0 || p.Ci < 1 || p.Ci > 64 || p.H < 1 || p.H > 512) return 1;
+  if (p.mode == 1 && (p.Co2 < 1 || p.Co2 > 4)) return 1;
+  const int no = p.mode == 1 ? p.Co2 : 1;   // dw2 rows of the backward
   if ((uintptr_t)x & 15) return 1;
   p.Cip = b2no_round_up(p.Ci, 8);
   p.Hp = b2no_round_up(p.H, 64);
@@ -546,10 +597,13 @@ int mlp_launch(MlpTc& p, const float* x, int batch, long pixels, cudaStream_t st
   if (mlp_tmem_cols(p) > 512) return 1;
   int dev = 0, max_smem = 0;
   B2NO_CHECK_CUDA(cudaGetDevice(&dev));
+  // cuTensorMapEncodeTiled (driver API) needs a current context; a thread whose first CUDA call is this one (autograd's
+  // backward thread, when every tensor it allocated came from the caching allocator's pool) has none yet
+  B2NO_CHECK_CUDA(cudaSetDevice(dev));
   B2NO_CHECK_CUDA(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
   MlpLayout L;
   for (p.S = 4; p.S >= 2; p.S--) {
-    L = mlp_layout(p);
+    L = mlp_layout(p, no);
     if ((int)L.total <= max_smem) break;
   }
   if (p.S < 2) return 1;
@@ -561,13 +615,17 @@ int mlp_launch(MlpTc& p, const float* x, int batch, long pixels, cudaStream_t st
   uint64_t str[3] = {4, (uint64_t)pixels * 4, (uint64_t)pixels * 4 * p.Ci};
   uint32_t box[3] = {128, (uint32_t)p.Cip, 1};
   if (make_tmap_f32(&tmx, x, 3, dims, str, box, CU_TENSOR_MAP_SWIZZLE_NONE)) return 1;
-#define MLP_LAUNCH(G, W, D)                                                                                              \
-  do {                                                                                                                   \
-    B2NO_CHECK_CUDA(cudaFuncSetAttribute(k_mlp_tc<G, W, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total)); \
-    k_mlp_tc<G, W, D><<<(unsigned)grid, kThreadsMlp, L.total, st>>>(tmx, p);                                            \
+#define MLP_LAUNCH(G, W, D, ...)                                                                                        \
+  do {                                                                                                                    \
+    B2NO_CHECK_CUDA(cudaFuncSetAttribute(k_mlp_tc<G, W, D, ##__VA_ARGS__>, cudaFuncAttributeMaxDynamicSharedMemorySize,   \
+                                         (int)L.total));                                                                  \
+    k_mlp_tc<G, W, D, ##__VA_ARGS__><<<(unsigned)grid, kThreadsMlp, L.total, st>>>(tmx, p);                             \
   } while (0)
   const bool gelu = p.act == B2NO_ACT_GELU;
-  if (p.mode == 1) { if (gelu) MLP_LAUNCH(true, true, false); else MLP_LAUNCH(false, true, false); }
+  if (p.mode == 1 && no == 2) { if (gelu) MLP_LAUNCH(true, true, false, 2); else MLP_LAUNCH(false, true, false, 2); }
+  else if (p.mode == 1 && no == 3) { if (gelu) MLP_LAUNCH(true, true, false, 3); else MLP_LAUNCH(false, true, false, 3); }
+  else if (p.mode == 1 && no == 4) { if (gelu) MLP_LAUNCH(true, true, false, 4); else MLP_LAUNCH(false, true, false, 4); }
+  else if (p.mode == 1) { if (gelu) MLP_LAUNCH(true, true, false); else MLP_LAUNCH(false, true, false); }
   else if (p.direct) { if (gelu) MLP_LAUNCH(true, false, true); else MLP_LAUNCH(false, false, true); }
   else { if (gelu) MLP_LAUNCH(true, false, false); else MLP_LAUNCH(false, false, false); }
 #undef MLP_LAUNCH
@@ -594,8 +652,8 @@ int b2no_tc_mlp_fwd(const float* x, const float* w1, const float* b1, const floa
   return rc;
 }
 
-// 1 when b2no_mlp_head_bwd has a kernel for this shape (mirrors the checks of mlp_launch)
-extern "C" int b2no_mlp_head_bwd_supported(int ci, int hidden, int64_t pixels) {
+// 1 when the backward has a kernel for this shape and `no` outputs (mirrors the checks of mlp_launch)
+static int mlp_bwd_supported(int ci, int hidden, int no, int64_t pixels) {
   if (!b2no_tc_available()) return 0;
   if (pixels < 128 || pixels % 128 != 0 || ci < 1 || ci > 64 || hidden < 1 || hidden > 512) return 0;
   MlpTc p;
@@ -605,8 +663,10 @@ extern "C" int b2no_mlp_head_bwd_supported(int ci, int hidden, int64_t pixels) {
   if (mlp_tmem_cols(p) > 512) return 0;
   int dev = 0, max_smem = 0;
   if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess) return 0;
-  return (int)mlp_layout(p).total <= max_smem ? 1 : 0;
+  return (int)mlp_layout(p, no).total <= max_smem ? 1 : 0;
 }
+
+extern "C" int b2no_mlp_head_bwd_supported(int ci, int hidden, int64_t pixels) { return mlp_bwd_supported(ci, hidden, 1, pixels); }
 
 extern "C" int64_t b2no_mlp_head_bwd_scratch_floats(int hidden) {
   if (hidden < 1) return B2NO_E_ARG;
@@ -630,6 +690,52 @@ extern "C" int b2no_mlp_head_bwd(const float* x, const float* w1, const float* b
   if (rc) return rc;
   b2no_tc_count_launch();
   k_sum_partials<<<(hidden + 31) / 32, 256, 0, st>>>(partial, dw2, grid, hidden);
+  B2NO_LAUNCH_CHECK();
+  return 0;
+}
+
+// ---- heads with 2..4 output channels (PINObserverFullField's plane_num * out_dim tail, pinobserver.py:230-232 / :257-273;
+// neuralop Projection with out_channels > 1, tfno.py:34-38) ----
+
+extern "C" int b2no_mlp_head_fwd_multi(const float* x, const float* w1, const float* b1, const float* w2, const float* b2, float* out,
+                                       int batch, int ci, int hidden, int out_channels, int64_t pixels, int b1_per_sample, int act,
+                                       void* stream) {
+  if (!x || !w1 || !w2 || !out || batch < 1 || ci < 1 || hidden < 1 || pixels < 1) return B2NO_E_ARG;
+  if (out_channels < 2 || out_channels > 4) return B2NO_E_UNSUPPORTED;
+  const int rc = b2no_tc_mlp_fwd(x, w1, b1, w2, b2, out, batch, ci, hidden, out_channels, (long)pixels, b1_per_sample, act,
+                                 (cudaStream_t)stream);
+  return rc == 1 ? B2NO_E_UNSUPPORTED : rc;
+}
+
+extern "C" int b2no_mlp_head_bwd_multi_supported(int ci, int hidden, int out_channels, int64_t pixels) {
+  if (out_channels < 2 || out_channels > 4) return 0;
+  return mlp_bwd_supported(ci, hidden, out_channels, pixels);
+}
+
+extern "C" int64_t b2no_mlp_head_bwd_multi_scratch_floats(int hidden, int out_channels) {
+  if (hidden < 1 || out_channels < 1) return B2NO_E_ARG;
+  return (int64_t)b2no_sm_count() * hidden * out_channels;
+}
+
+extern "C" int b2no_mlp_head_bwd_multi(const float* x, const float* w1, const float* b1, const float* w2, const float* g, float* gx,
+                                       float* gz, float* dw2, float* partial, int batch, int ci, int hidden, int out_channels,
+                                       int64_t pixels, int b1_per_sample, int act, const float* dact_z, int dact, void* stream) {
+  if (!x || !w1 || !w2 || !g || !gx || !dw2 || !partial || batch < 1 || ci < 1 || hidden < 1 || pixels < 1) return B2NO_E_ARG;
+  if (out_channels < 2 || out_channels > 4) return B2NO_E_UNSUPPORTED;
+  cudaStream_t st = (cudaStream_t)stream;
+  MlpTc p;
+  memset(&p, 0, sizeof(p));
+  p.npass = b2no_tc_passes();
+  p.B = batch; p.Ci = ci; p.H = hidden; p.Co2 = out_channels; p.mode = 1; p.act = act; p.b1_per_sample = b1_per_sample;
+  p.w1 = w1; p.b1 = b1; p.w2 = w2; p.g = g; p.out = gx; p.gz = gz; p.dw2_partial = partial;
+  p.dz = dact_z; p.dact = dact_z ? dact : 0;
+  int grid = 0;
+  const int rc = mlp_launch(p, x, batch, (long)pixels, st, &grid);
+  if (rc == 1) return B2NO_E_UNSUPPORTED;
+  if (rc) return rc;
+  b2no_tc_count_launch();
+  const int n = out_channels * hidden;   // partial rows: (o, j) of every CTA
+  k_sum_partials<<<(n + 31) / 32, 256, 0, st>>>(partial, dw2, grid, n);
   B2NO_LAUNCH_CHECK();
   return 0;
 }

@@ -352,9 +352,58 @@ class MlpHeadFn(torch.autograd.Function):
                 dw2.reshape(ctx.shapes[2]) if need_w2 else None, db2, None)
 
 
+class MlpHeadMultiFn(torch.autograd.Function):
+    """out[:, o] = b2[o] + w2[o] . act(W1 x + b1) for 2..4 outputs: PINObserverFullField's tail (plane_num * out_dim channels,
+    pinobserver.py:230-232) and Projection with out_channels > 1 (tfno.py:34-38).  Like MlpHeadFn, the hidden tensor is never
+    stored: the backward recomputes it on the tensor cores (csrc/tc_mlp.cu), emits gx and dW2 directly and writes
+    gz = act'(z1) sum_o g[o] w2[o] once for the weight-gradient kernel."""
+
+    @staticmethod
+    def forward(ctx, x, w1, b1, w2, b2, act):
+        ops._require_cuda(x)
+        x = _contig(x.float())
+        w1m = _contig(w1.detach().reshape(w1.shape[0], -1).float())
+        w2m = _contig(w2.detach().reshape(w2.shape[0], -1).float())
+        b1c = None if b1 is None else _contig(b1.detach().float())
+        out = ops.mlp_head_fwd_multi(x, w1m, b1c, w2m, None if b2 is None else _contig(b2.detach().float()), act)
+        if out is None:
+            raise RuntimeError("mlp_head: the multi-output head kernel declined a shape mlp_head_fused_available accepted")
+        ctx.act = act
+        ctx.shapes = (tuple(w1.shape), None if b1 is None else tuple(b1.shape), tuple(w2.shape),
+                      None if b2 is None else tuple(b2.shape))
+        ctx.save_for_backward(x, w1m, b1c, w2m)
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        x, w1m, b1c, w2m = ctx.saved_tensors
+        g = _contig(g.float())
+        need_x, need_w1, need_b1, need_w2, need_b2 = ctx.needs_input_grad[:5]
+        res = ops.mlp_head_bwd_multi(x, w1m, b1c, w2m, g, ctx.act, want_gz=need_w1 or need_b1)
+        if res is None:
+            raise RuntimeError("mlp_head backward: shape lost its tensor-core kernel between forward and backward")
+        gx, gz, dw2 = res
+        dw1 = db1 = None
+        if need_w1 or need_b1:
+            per_sample = b1c is not None and b1c.dim() == 2
+            dw1, db1 = ops.pw_wgrad(gz, x, need_bias=need_b1 and not per_sample)
+            dw1 = dw1.reshape(ctx.shapes[0])
+            if need_b1 and per_sample:
+                db1 = gz.sum(dim=tuple(range(2, gz.dim())))
+            if db1 is not None:
+                db1 = db1.reshape(ctx.shapes[1])
+        db2 = g.sum(dim=[0] + list(range(2, g.dim()))).reshape(ctx.shapes[3]) if need_b2 else None
+        return (gx if need_x else None, dw1 if need_w1 else None, db1 if need_b1 else None,
+                dw2.reshape(ctx.shapes[2]) if need_w2 else None, db2, None)
+
+
 def mlp_head_fused_available(x, w1, w2, b1, needs_grad: bool) -> bool:
-    """True when mlp_head() runs the fused tensor-core head for these operands (the hidden tensor is never materialised)."""
-    if not x.is_cuda or w2.reshape(-1, w1.shape[0]).shape[0] != 1 or (b1 is not None and b1.dim() > 2):
+    """True when mlp_head() runs the fused tensor-core head for these operands (the hidden tensor is never materialised).
+    One output: the kernels of MlpHeadFn; 2..4 outputs: those of MlpHeadMultiFn, in training and inference alike."""
+    n_out = w2.reshape(-1, w1.shape[0]).shape[0]
+    if 2 <= n_out <= 4 and (b1 is None or b1.dim() <= 2):
+        return ops.mlp_head_multi_supported(x, w1.shape[0], n_out)
+    if not x.is_cuda or n_out != 1 or (b1 is not None and b1.dim() > 2):
         return False
     if needs_grad:
         return bool(ops.mlp_head_bwd_supported(x.shape[1], w1.shape[0], math.prod(x.shape[2:]))) and x.data_ptr() % 16 == 0
@@ -362,12 +411,23 @@ def mlp_head_fused_available(x, w1, w2, b1, needs_grad: bool) -> bool:
 
 
 def mlp_head(x, w1, b1, w2, b2, act="gelu"):
-    """Projection head Ci -> hidden -> act -> 1 (tfno.py:34-38).  The fused kernels never materialise the hidden
-    tensor in the forward; shapes without a fused kernel compose two pointwise convs (hidden saved for backward)."""
+    """Projection head Ci -> hidden -> act -> O (tfno.py:34-38).  For O = 1..4 the fused kernels never materialise the
+    hidden tensor in the forward; other O and shapes without a fused kernel compose two pointwise convs (hidden saved for
+    backward)."""
     ops._require_cuda(x, w1, b1, w2, b2)
     needs_grad = torch.is_grad_enabled() and any(
         t is not None and t.requires_grad for t in (x, w1, b1, w2, b2))
     if mlp_head_fused_available(x, w1, w2, b1, needs_grad):
+        if w2.reshape(-1, w1.shape[0]).shape[0] > 1:
+            if needs_grad:
+                return MlpHeadMultiFn.apply(x, w1, b1, w2, b2, act)
+            out = ops.mlp_head_fwd_multi(_contig(x.float()), _contig(w1.reshape(w1.shape[0], -1).float()),
+                                         None if b1 is None else _contig(b1.float()),
+                                         _contig(w2.reshape(w2.shape[0], -1).float()),
+                                         None if b2 is None else _contig(b2.float()), act)
+            if out is None:
+                raise RuntimeError("mlp_head: the multi-output head kernel declined a shape mlp_head_fused_available accepted")
+            return out
         if needs_grad:
             return MlpHeadFn.apply(x, w1, b1, w2, b2, act)
         return ops.mlp_head_fwd(_contig(x.float()), _contig(w1.reshape(w1.shape[0], -1).float()),

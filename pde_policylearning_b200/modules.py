@@ -852,10 +852,10 @@ def _pino_trunk_forward(x, re, fc0, mnet1, sp_convs, ws, mnet2, fc1, fc2, act_na
     szp = sz + num_pad[0] + num_pad[1]
     needs_grad = torch.is_grad_enabled() and (h.requires_grad or w1.requires_grad)
     h = h if h.is_contiguous() else h.contiguous()
-    if fc2.out_features == 1 and Fn.mlp_head_fused_available(h, w1, fc2.weight, None, needs_grad):
-        # fused head (training and inference): the per-sample bias carries the Reynolds term, the fc_dim-wide hidden
-        # tensor is never materialised in the forward; autograd reaches A / B / bias of MultiplicativeNet2 and fc1
-        # through the folded w1 / per-sample b1
+    if Fn.mlp_head_fused_available(h, w1, fc2.weight, None, needs_grad):
+        # fused head (training and inference, out_dim 1..4 -- PINObserverFullField emits plane_num * out_dim): the
+        # per-sample bias carries the Reynolds term, the fc_dim-wide hidden tensor is never materialised in the forward;
+        # autograd reaches A / B / bias of MultiplicativeNet2 and fc1 through the folded w1 / per-sample b1
         out = Fn.mlp_head(h, w1, b1[None, :] + re @ wre.t(), fc2.weight, fc2.bias, act_name)
     else:
         re_map = re.reshape(B, 1, 1, 1, 1).expand(B, 1, sx, sy, szp).contiguous()

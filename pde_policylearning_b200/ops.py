@@ -431,6 +431,51 @@ def mlp_head_bwd_fused(x, w1, b1, w2, g, act="gelu", dact_z=None, dact=None):
     return gx, grads[:n].view(hidden, ci), grads[n:n + hidden], grads[n + hidden:n + 2 * hidden], grads[n + 2 * hidden:]
 
 
+def mlp_head_multi_supported(x: torch.Tensor, hidden: int, out_channels: int) -> bool:
+    """True when the fused head with out_channels = 2..4 runs for x, forward and backward (b2no_mlp_head_bwd_multi_supported;
+    its shapes are a subset of the forward's): a CUDA tensor, 16-byte aligned for the tensor-map load."""
+    if not x.is_cuda or x.data_ptr() % 16 != 0:
+        return False
+    return bool(_lib.lib().b2no_mlp_head_bwd_multi_supported(x.shape[1], hidden, out_channels, math.prod(x.shape[2:])))
+
+
+def mlp_head_fwd_multi(x, w1, b1, w2, b2, act="gelu") -> Optional[torch.Tensor]:
+    """Ci -> hidden -> act -> O head, O = w2.shape[0] in 2..4, without the hidden tensor (b2no_mlp_head_fwd_multi).
+    Returns (B, O, *grid), or None -- with nothing computed -- when the shape has no kernel."""
+    B, ci = x.shape[:2]
+    grid = tuple(x.shape[2:])
+    hidden, O = w1.shape[0], w2.shape[0]
+    per_sample = b1 is not None and b1.dim() == 2
+    out = torch.empty((B, O) + grid, dtype=torch.float32, device=x.device)
+    rc = _lib.lib().b2no_mlp_head_fwd_multi(_ptr(x), _ptr(w1), _ptr(b1), _ptr(w2), _ptr(b2), _ptr(out), B, ci, hidden, O,
+                                            math.prod(grid), 1 if per_sample else 0, ACT[act], _stream())
+    if rc == -2:
+        return None
+    check(rc, "mlp_head_fwd_multi")
+    return out
+
+
+def mlp_head_bwd_multi(x, w1, b1, w2, g, act="gelu", want_gz=True, dact_z=None, dact=None):
+    """Input-gradient half of the backward of the Ci -> hidden -> act -> O head (b2no_mlp_head_bwd_multi), g (B, O, *grid).
+    Returns (gx, gz | None, dw2 (O, hidden)) or None when the shape has no tensor-core kernel."""
+    B, ci = x.shape[:2]
+    grid = tuple(x.shape[2:])
+    hidden, O = w1.shape[0], w2.shape[0]
+    L = _lib.lib()
+    per_sample = b1 is not None and b1.dim() == 2
+    gx = torch.empty_like(x)
+    gz = torch.empty((B, hidden) + grid, dtype=torch.float32, device=x.device) if want_gz else None
+    dw2 = torch.empty((O, hidden), dtype=torch.float32, device=x.device)
+    partial = torch.empty(int(L.b2no_mlp_head_bwd_multi_scratch_floats(hidden, O)), dtype=torch.float32, device=x.device)
+    rc = L.b2no_mlp_head_bwd_multi(_ptr(x), _ptr(w1), _ptr(b1), _ptr(w2), _ptr(g), _ptr(gx), _ptr(gz), _ptr(dw2), _ptr(partial),
+                                   B, ci, hidden, O, math.prod(grid), 1 if per_sample else 0, ACT[act], _ptr(dact_z),
+                                   ACT[dact] if dact_z is not None else 0, _stream())
+    if rc == -2:
+        return None
+    check(rc, "mlp_head_bwd_multi")
+    return gx, gz, dw2
+
+
 def rno_gate_fwd(z, z2, hh, h):
     out = torch.empty_like(h)
     check(_lib.lib().b2no_rno_gate_fwd(_ptr(z), _ptr(z2), _ptr(hh), _ptr(h), _ptr(out), h.numel(), _stream()), "gate")
