@@ -147,6 +147,24 @@ int b2no_mix(const b2no_plan* plan, int mode, const float* in, const b2no_weight
 int b2no_mix_dw(const b2no_plan* plan, const float* xh, const float* gyh, const b2no_weights* dw,
                 int batch, int ci, int co, int accumulate, void* stream);
 
+/* ---- normalisation of a spectral convolution's output (fno_block.py:94-105,142-150) ------------- */
+/* GroupNorm(groups) of s = s_i Re IDFT_trunc(Yh) + bias[c] over (channels of the group, output grid), with optional per-channel
+ * affine gamma / beta; InstanceNorm is groups = channels.  Computed on the kept-mode spectrum (layout 0), which is what the
+ * inverse transform then turns into the normalised activation with NO bias in its epilogue:
+ *   out[b,c,k] = gamma[c] rstd[b,g] Yh[b,c,k]   (k != 0);   out[b,c,0] = (gamma[c] (mu[b,c] - mu[b,g]) rstd[b,g] + beta[c]) / s_i
+ * with mu / var the exact mean and variance of s over the grid.  bias may be NULL; gamma and beta are both NULL or both
+ * given; eps > 0.  stats receives 2 * batch * (channels + groups) floats, [(mu, var) per (b, c) | (mu, rstd) per (b, g)], for
+ * the backward.  Returns B2NO_E_UNSUPPORTED for a mode-major plan or one whose output grid differs from its transform size. */
+int b2no_spec_norm_fwd(const b2no_plan* plan, const float* spec, const float* bias, const float* gamma, const float* beta,
+                       float eps, float* out, float* stats, int batch, int channels, int groups, void* stream);
+/* Its backward: gout = dL/dYh from gspec = dL/dout (b2no_dft_forward(plan, 1, .) of the activation gradient), spec and stats of
+ * the forward.  dbias, dgamma, dbeta (channels each, any may be NULL) are summed over the batch in a fixed order.
+ * scratch: b2no_spec_norm_bwd_scratch_floats(batch, channels) floats. */
+int64_t b2no_spec_norm_bwd_scratch_floats(int batch, int channels);
+int b2no_spec_norm_bwd(const b2no_plan* plan, const float* spec, const float* gspec, const float* stats, const float* gamma,
+                       float* gout, float* dbias, float* dgamma, float* dbeta, float* scratch, int batch, int channels,
+                       int groups, void* stream);
+
 /* ---- pointwise kernels -------------------------------------------------------------------------- */
 /* gz = gy * act'(z)  (elementwise, n floats) */
 int b2no_act_bwd(const float* gy, const float* z, float* gz, int64_t n, int act, void* stream);

@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # B2NO_LIB: load another build, e.g. the parent commit's, for A/B runs in one call
 LIB_PATH = os.environ.get("B2NO_LIB") or os.path.join(_HERE, "libb2no.so")
 CSRC = os.path.join(_HERE, "csrc")
-SOURCES = ["plan.cu", "spectral.cu", "pointwise.cu", "tc_pointwise.cu", "tc_wgrad.cu", "tc_mlp.cu", "tc_head_bwd.cu", "tc_dft.cu", "tc_mix.cu", "tc_peak.cu", "pino_loss.cu", "optim.cu"]
+SOURCES = ["plan.cu", "spectral.cu", "pointwise.cu", "tc_pointwise.cu", "tc_wgrad.cu", "tc_mlp.cu", "tc_head_bwd.cu", "tc_dft.cu", "tc_mix.cu", "tc_peak.cu", "pino_loss.cu", "optim.cu", "spec_norm.cu"]
 
 MAX_DIM = 3
 NORM = {"backward": 0, "forward": 1, "ortho": 2}
@@ -105,6 +105,10 @@ def lib():
     L.b2no_mix.argtypes = [vp, i32, vp, C.POINTER(Weights), vp, i32, i32, i32, i32, vp]
     L.b2no_mix_dw.argtypes = [vp, vp, vp, C.POINTER(Weights), i32, i32, i32, i32, vp]
     L.b2no_act_bwd.argtypes = [vp, vp, vp, i64, i32, vp]
+    L.b2no_spec_norm_fwd.argtypes = [vp, vp, vp, vp, vp, C.c_float, vp, vp, i32, i32, i32, vp]
+    L.b2no_spec_norm_bwd_scratch_floats.restype = i64
+    L.b2no_spec_norm_bwd_scratch_floats.argtypes = [i32, i32]
+    L.b2no_spec_norm_bwd.argtypes = [vp] * 10 + [i32, i32, i32, vp]
     L.b2no_pw_wgrad_scratch_floats.restype = i64
     L.b2no_pw_wgrad_scratch_floats.argtypes = [i32, i32]
     L.b2no_pw_wgrad.argtypes = [vp, vp, vp, vp, vp, i32, i32, i32, i64, vp]
@@ -150,6 +154,7 @@ EXPORTS = [
     "b2no_plan_create", "b2no_plan_destroy", "b2no_plan_kept", "b2no_plan_layout_supported", "b2no_plan_workspace_floats",
     "b2no_set_tensor_core_mode", "b2no_set_precision", "b2no_tensor_core_launches", "b2no_kernel_launches",
     "b2no_dft_forward", "b2no_dft_inverse", "b2no_mix", "b2no_mix_dw",
+    "b2no_spec_norm_fwd", "b2no_spec_norm_bwd_scratch_floats", "b2no_spec_norm_bwd",
     "b2no_act_bwd", "b2no_pw_wgrad_scratch_floats", "b2no_pw_wgrad", "b2no_dft_inverse_wgrad", "b2no_mlp_head_fwd", "b2no_mlp_head_bwd_scratch_floats", "b2no_mlp_head_bwd_supported", "b2no_mlp_head_bwd",
     "b2no_mlp_head_bwd_fused_scratch_floats", "b2no_mlp_head_bwd_fused_supported", "b2no_mlp_head_bwd_fused",
     "b2no_mlp_head_fwd_multi", "b2no_mlp_head_bwd_multi_supported", "b2no_mlp_head_bwd_multi_scratch_floats",

@@ -72,8 +72,11 @@ def _convert_pino_conv2d(ref) -> nn.Module:
 
 
 def _convert_fno_blocks(ref):
-    ok = (ref.mlp is None and ref.norm is None and not ref.preactivation and ref.fno_skip == "linear"
+    ok = (ref.mlp is None and not ref.preactivation and ref.fno_skip == "linear"
           and ref.output_scaling_factor is None and isinstance(ref.convs, M.SpectralConv))
+    # instance / group norms run on the spectrum (M.norm_args); any other norm keeps the block in torch
+    if ok and ref.norm is not None:
+        ok = len(ref.norm) >= ref.n_layers and all(M.norm_args(m, ref.out_channels) is not None for m in ref.norm)
     if not ok:
         return None
     new = M.FNOBlocks.__new__(M.FNOBlocks)
@@ -82,9 +85,9 @@ def _convert_fno_blocks(ref):
               "n_layers", "joint_factorization", "non_linearity", "fno_skip", "mlp_skip", "fft_norm"):
         setattr(new, k, getattr(ref, k))
     new.mlp = None
-    new.norm = None
     new.convs = ref.convs
     new.fno_skips = ref.fno_skips
+    new.norm = ref.norm              # the same norm modules (and Parameters), or None
     new.train(ref.training)
     return new
 

@@ -74,6 +74,9 @@ struct b2no_plan {
   float2* m_adjfwd[2];  // [K_j][nin_j]    conj(m_fwd)^T
   int* row_corner[2];   // [K_j] 0 = low corner, 1 = high corner
   int* row_local[2];    // [K_j] index inside the corner's weight
+  // [total kept modes] (mirror, c) of the spectral normalisation (spec_norm.cu): c = c(k_d) of the inverse (0, 1, 2);
+  // mirror = flat index of the kept mode at frequency -k when c == 1 and that mode is kept, else -1
+  int2* norm_tab;
 };
 
 // ---- kept-mode bookkeeping shared by the mixing kernels (spectral.cu, tc_mix.cu) -----------------------------------

@@ -234,6 +234,41 @@ extern "C" int b2no_plan_create(const b2no_geom* g, b2no_plan** out) {
     if ((rc = upload(&p->row_corner[j], rcorner))) return rc;
     if ((rc = upload(&p->row_local[j], rlocal))) return rc;
   }
+  // ---- per-mode table of the spectral normalisation (spec_norm.cu) ----------------------------
+  {
+    std::vector<Row> rows[B2NO_MAX_DIM];
+    std::vector<int> pos[B2NO_MAX_DIM];     // frequency -> kept row, -1 when not kept (two-sided dims)
+    for (int j = 0; j < d; j++) {
+      rows[j] = kept_rows(g->nfft[j], g->half[j], j == d - 1);
+      if (j == d - 1) continue;
+      pos[j].assign(g->nfft[j], -1);
+      for (int r = 0; r < (int)rows[j].size(); r++) pos[j][rows[j][r].f] = r;
+    }
+    int kt = 1;
+    for (int j = 0; j < d; j++) kt *= p->K[j];
+    std::vector<int2> tab(kt);
+    const int N = g->nfft[d - 1], Np = g->nout[d - 1];
+    for (int k = 0; k < kt; k++) {
+      int idx[B2NO_MAX_DIM], rem = k;
+      for (int j = d - 1; j >= 0; j--) { idx[j] = rem % p->K[j]; rem /= p->K[j]; }
+      const int f = idx[d - 1];
+      int c = 2;                                            // c(k_d) exactly as the last-dim table T_out above
+      if (f == 0 || (Np % 2 == 0 && f == Np / 2)) c = 1;
+      if (f >= Np / 2 + 1 || f >= N / 2 + 1) c = 0;
+      int mirror = -1;
+      if (c == 1) {
+        mirror = 0;
+        for (int j = 0; j < d - 1 && mirror >= 0; j++) {
+          const int Nj = g->nfft[j], r = pos[j][(Nj - rows[j][idx[j]].f) % Nj];
+          mirror = r < 0 ? -1 : mirror * p->K[j] + r;
+        }
+        if (mirror >= 0) mirror = mirror * p->K[d - 1] + f;
+      }
+      tab[k] = make_int2(mirror, c);
+    }
+    int rc;
+    if ((rc = upload(&p->norm_tab, tab))) return rc;
+  }
   // ---- tensor-core forward-DFT operand images (2-D; tc_dft.cu) --------------------------------
   for (int which = 0; which < 2; which++) {
     b2no_tc_fwd_tables& tf = p->tcf[which];
@@ -297,6 +332,7 @@ extern "C" int b2no_plan_destroy(b2no_plan* p) {
   cudaFree(p->t_out);
   cudaFree(p->tc[0].timg);
   cudaFree(p->tc[1].timg);
+  cudaFree(p->norm_tab);
   for (int w = 0; w < 2; w++) { cudaFree(p->tcf[w].tb); cudaFree(p->tcf[w].mimg); }
   for (int j = 0; j < 2; j++) {
     cudaFree(p->m_fwd[j]); cudaFree(p->m_inv[j]); cudaFree(p->m_adjinv[j]); cudaFree(p->m_adjfwd[j]);

@@ -38,7 +38,7 @@ class SpectralBlockFn(torch.autograd.Function):
     spectral convolutions (spectral_convolution.py:303-347, rno.py:60-77, basics.py:114-143)."""
 
     @staticmethod
-    def forward(ctx, x, bias, pw_w, geom: SpecGeom, act, *corners):
+    def forward(ctx, x, bias, pw_w, geom: SpecGeom, act, norm, gamma, beta, *corners):
         ops._require_cuda(x)
         x = _contig(x.float())
         plan = get_plan(geom, x.device)
@@ -49,6 +49,11 @@ class SpectralBlockFn(torch.autograd.Function):
         det = [c.detach() for c in corners]
         xh = ops.dft_forward(plan, 0, x)
         yh = ops.mix(plan, 0, xh, det, ci, co)
+        normed = None
+        if norm is not None:
+            # Norm(conv + bias) on the spectrum: the inverse then runs without the bias
+            gam, bet = _norm_affine(gamma, beta)
+            normed = ops.spec_norm_fwd(plan, yh, _vec(bias), gam, bet, norm[0], norm[1])
         need_z = act not in (None, "none") and any(ctx.needs_input_grad)
         grid = plan.geom.nout
         z = torch.empty((B, co) + tuple(grid), dtype=torch.float32, device=x.device) if need_z else None
@@ -57,19 +62,25 @@ class SpectralBlockFn(torch.autograd.Function):
             if tuple(plan.geom.nout) != tuple(plan.geom.nin):
                 raise NotImplementedError("fused 1x1 skip needs matching input/output grids")
             pw2d = _contig(pw_w.detach().reshape(pw_w.shape[0], -1).float())
-        epi = ops.make_epilogue(bias=None if bias is None else _contig(bias.detach().reshape(-1).float()),
+        epi = ops.make_epilogue(bias=None if (bias is None or norm is not None) else _vec(bias),
                                 pw_w=pw2d, pw_x=x if pw2d is not None else None, preact=z, act=act)
-        y = ops.dft_inverse(plan, 0, yh, epi)
-        ctx.geom, ctx.act = geom, act
+        y = ops.dft_inverse(plan, 0, yh if normed is None else normed[0], epi)
+        ctx.geom, ctx.act, ctx.norm = geom, act, norm
         ctx.has_bias, ctx.has_pw = bias is not None, pw_w is not None
         ctx.pw_shape = None if pw_w is None else tuple(pw_w.shape)
         ctx.bias_shape = None if bias is None else tuple(bias.shape)
-        ctx.save_for_backward(x, xh, z, pw2d, *det)
+        if normed is None:
+            ctx.save_for_backward(x, xh, z, pw2d, *det)
+        else:
+            ctx.save_for_backward(x, xh, z, pw2d, yh, normed[1], gam, *det)
         return y
 
     @staticmethod
     def backward(ctx, gy):
-        x, xh, z, pw2d, *det = ctx.saved_tensors
+        if ctx.norm is None:
+            x, xh, z, pw2d, *det = ctx.saved_tensors
+        else:
+            x, xh, z, pw2d, yh, stats, gam, *det = ctx.saved_tensors
         geom, act = ctx.geom, ctx.act
         plan = get_plan(geom, x.device)
         B, ci = x.shape[:2]
@@ -77,9 +88,16 @@ class SpectralBlockFn(torch.autograd.Function):
         gy = _contig(gy.float())
         gz = ops.act_bwd(gy, z, act) if z is not None else gy
         need_x, need_b, need_pw = ctx.needs_input_grad[0], ctx.needs_input_grad[1], ctx.needs_input_grad[2]
-        need_w = any(ctx.needs_input_grad[5:])
+        need_w = any(ctx.needs_input_grad[8:])
         gyh = ops.dft_forward(plan, 1, gz)
-        dbias = dpw = dx = None
+        dbias = dpw = dx = dgamma = dbeta = None
+        if ctx.norm is not None:
+            # the bias only enters through the norm's statistics: its gradient comes from the norm backward alone
+            need_affine = ctx.needs_input_grad[6] or ctx.needs_input_grad[7]
+            gyh, db, dgamma, dbeta = ops.spec_norm_bwd(plan, yh, gyh, stats, gam, ctx.norm[0], need_b, need_affine)
+            if need_b:
+                dbias = db.reshape(ctx.bias_shape)
+            need_b = False
         dcorners: List[Optional[torch.Tensor]] = [None] * len(det)
         if need_w:
             dcorners = ops.mix_dw(plan, xh, gyh, det, needs_zero=_geom_has_overlap(geom))
@@ -99,11 +117,28 @@ class SpectralBlockFn(torch.autograd.Function):
             # dbias[o] = sum_{b,n} gz = DC mode of the (scaled) truncated DFT: gYh[b,o,0..0] = s_i * sum_n gz
             dc = gyh.reshape(B, co, -1)[:, :, 0].real.sum(dim=0) / plan.s_i
             dbias = dc.reshape(ctx.bias_shape)
-        return (dx, dbias, dpw, None, None) + tuple(dcorners)
+        return (dx, dbias, dpw, None, None, None, dgamma, dbeta) + tuple(dcorners)
 
 
-def spectral_block(x, corners: Sequence[torch.Tensor], geom: SpecGeom, bias=None, pw_weight=None, act=None):
-    return SpectralBlockFn.apply(x, bias, pw_weight, geom, act, *corners)
+def _vec(t: Optional[torch.Tensor]) -> Optional[torch.Tensor]:
+    return None if t is None else _contig(t.detach().reshape(-1).float())
+
+
+def _norm_affine(gamma, beta):
+    """Per-channel affine parameters of a norm as the kernels take them: both given, or both None."""
+    if (gamma is None) != (beta is None):
+        raise NotImplementedError("a norm with only one of weight / bias has no native kernel")
+    return _vec(gamma), _vec(beta)
+
+
+def spectral_block(x, corners: Sequence[torch.Tensor], geom: SpecGeom, bias=None, pw_weight=None, act=None, norm=None):
+    """norm: None, or (groups, eps, gamma, beta) -- y = act(GroupNorm(spectral_conv(x) + bias) + pw_weight x), the
+    normalisation applied to the kept-mode spectrum (ops.spec_norm_fwd); instance norm is groups = channels and gamma / beta
+    are None without affine parameters."""
+    if norm is None:
+        return SpectralBlockFn.apply(x, bias, pw_weight, geom, act, None, None, None, *corners)
+    groups, eps, gamma, beta = norm
+    return SpectralBlockFn.apply(x, bias, pw_weight, geom, act, (int(groups), float(eps)), gamma, beta, *corners)
 
 
 class FNOStackFn(torch.autograd.Function):
@@ -114,14 +149,19 @@ class FNOStackFn(torch.autograd.Function):
 
     bias_all = the (n_layers, Co, 1, ...) bias parameter of the conv stack (spectral_convolution.py:271-272), taken whole
     so that its gradient is written once by the weight-gradient kernels instead of being assembled from per-layer
-    slices; params = for each layer: pw_w (Co, Ci, 1...) | n_corners corner tensors."""
+    slices; params = for each layer: pw_w (Co, Ci, 1...) | n_corners corner tensors [| norm weight | norm bias].
+
+    norm = None, or (groups, eps, affine): every layer is y = act_l(GroupNorm_l(spectral_conv_l(x) + bias_l) + skip_l x)
+    (fno_block.py:142-150), the norm applied to the kept-mode spectrum between the mixing and the inverse transform
+    (ops.spec_norm_fwd); with affine the layer's params end with the norm's weight and bias."""
 
     @staticmethod
-    def forward(ctx, x, geom: SpecGeom, acts, n_corners, bias_all, *params):
+    def forward(ctx, x, geom: SpecGeom, acts, n_corners, norm, bias_all, *params):
         ops._require_cuda(x)
         x = _contig(x.float())
         plan = get_plan(geom, x.device)
-        per = 1 + n_corners
+        n_aff = 2 if (norm is not None and norm[2]) else 0
+        per = 1 + n_corners + n_aff
         L = len(params) // per
         need_grad = any(ctx.needs_input_grad)
         saved, meta = [], []
@@ -129,7 +169,7 @@ class FNOStackFn(torch.autograd.Function):
         b2d = _contig(bias_all.detach().reshape(L, -1).float())
         for l in range(L):
             pw_w = params[l * per]
-            det = [c.detach() for c in params[l * per + 1:(l + 1) * per]]
+            det = [c.detach() for c in params[l * per + 1:l * per + 1 + n_corners]]
             B, ci = cur.shape[:2]
             co = det[0].shape[1]
             xh = ops.dft_forward(plan, 0, cur)
@@ -138,26 +178,35 @@ class FNOStackFn(torch.autograd.Function):
             need_z = act not in (None, "none") and need_grad
             z = torch.empty((B, co) + tuple(plan.geom.nout), dtype=torch.float32, device=x.device) if need_z else None
             pw2d = _contig(pw_w.detach().reshape(pw_w.shape[0], -1).float())
-            epi = ops.make_epilogue(bias=b2d[l], pw_w=pw2d, pw_x=cur, preact=z, act=act)
-            y = ops.dft_inverse(plan, 0, yh, epi)
+            if norm is None:
+                epi = ops.make_epilogue(bias=b2d[l], pw_w=pw2d, pw_x=cur, preact=z, act=act)
+                y = ops.dft_inverse(plan, 0, yh, epi)
+            else:
+                gam, bet = (_vec(params[(l + 1) * per - 2]), _vec(params[(l + 1) * per - 1])) if n_aff else (None, None)
+                yhn, stats = ops.spec_norm_fwd(plan, yh, b2d[l], gam, bet, norm[0], norm[1])
+                epi = ops.make_epilogue(pw_w=pw2d, pw_x=cur, preact=z, act=act)
+                y = ops.dft_inverse(plan, 0, yhn, epi)
+                det = [yh, stats, gam if gam is not None else cur.new_empty(0)] + det
             saved += [cur, xh, z if z is not None else cur.new_empty(0), pw2d] + det
             meta.append((tuple(pw_w.shape), ci, co, need_z))
             cur = y
-        ctx.geom, ctx.acts, ctx.n_corners, ctx.meta = geom, acts, n_corners, meta
+        ctx.geom, ctx.acts, ctx.n_corners, ctx.meta, ctx.norm = geom, acts, n_corners, meta, norm
         ctx.bias_shape = tuple(bias_all.shape)
         ctx.save_for_backward(*saved)
         return cur
 
     @staticmethod
     def backward(ctx, gy):
-        geom, acts, nc, meta = ctx.geom, ctx.acts, ctx.n_corners, ctx.meta
+        geom, acts, nc, meta, norm = ctx.geom, ctx.acts, ctx.n_corners, ctx.meta, ctx.norm
         saved = ctx.saved_tensors
-        per_s = 4 + nc
+        nn_ = 0 if norm is None else 3                 # saved per layer with a norm: yh, stats, gamma
+        n_aff = 2 if (norm is not None and norm[2]) else 0
+        per_s = 4 + nn_ + nc
         L = len(meta)
         plan = get_plan(geom, gy.device)
-        per = 1 + nc
+        per = 1 + nc + n_aff
         grads = [None] * (L * per)
-        need_bias = ctx.needs_input_grad[4]
+        need_bias = ctx.needs_input_grad[5]
         dbias = gy.new_empty((L, meta[0][2])) if need_bias else None
         g = _contig(gy.float())
         # top layer: gradient w.r.t. its pre-activation
@@ -165,16 +214,25 @@ class FNOStackFn(torch.autograd.Function):
             g = ops.act_bwd(g, saved[(L - 1) * per_s + 2], acts[L - 1])
         for l in range(L - 1, -1, -1):
             x, xh, _, pw2d = saved[l * per_s: l * per_s + 4]
-            det = list(saved[l * per_s + 4: (l + 1) * per_s])
+            det = list(saved[l * per_s + 4 + nn_: (l + 1) * per_s])
             pw_shape, ci, co, _ = meta[l]
-            need = ctx.needs_input_grad[5 + l * per: 5 + (l + 1) * per]
+            need = ctx.needs_input_grad[6 + l * per: 6 + (l + 1) * per]
             gyh = ops.dft_forward(plan, 1, g)
-            if any(need[1:]):
+            # with a norm, dbias[l] comes from the norm backward; the 1x1 weight-gradient pass computes dWp only
+            wg_bias = need_bias and norm is None
+            if norm is not None:
+                yh, stats, gam = saved[l * per_s + 4: l * per_s + 7]
+                gyh, _, dgam, dbet = ops.spec_norm_bwd(plan, yh, gyh, stats, gam if n_aff else None, norm[0], need_bias,
+                                                       n_aff > 0 and any(need[1 + nc:]),
+                                                       db_out=dbias[l] if need_bias else None)
+                if n_aff:
+                    grads[(l + 1) * per - 2], grads[(l + 1) * per - 1] = dgam, dbet
+            if any(need[1:1 + nc]):
                 dcs = ops.mix_dw(plan, xh, gyh, det, needs_zero=_geom_has_overlap(geom))
                 for j in range(nc):
                     grads[l * per + 1 + j] = dcs[j]
-            need_wgrad = need_bias or need[0]
-            db_out = dbias[l] if need_bias else None
+            need_wgrad = wg_bias or need[0]
+            db_out = dbias[l] if wg_bias else None
             fused = None
             if l > 0 or ctx.needs_input_grad[0]:
                 gxh = ops.mix(plan, 1, gyh, det, ci, co)
@@ -183,29 +241,39 @@ class FNOStackFn(torch.autograd.Function):
                                         dact=acts[l - 1] if zprev is not None else None)
                 # the dx pass reads g tile by tile anyway: it also computes dWp and dbias[l] when it can
                 if need_wgrad and _fused_wgrad_ok(g):
-                    fused = ops.dft_inverse_wgrad(plan, 1, gxh, epi, x, need_bias=need_bias, db_out=db_out)
+                    fused = ops.dft_inverse_wgrad(plan, 1, gxh, epi, x, need_bias=wg_bias, db_out=db_out)
                 if fused is None:
                     if need_wgrad:
-                        dpw, _ = ops.pw_wgrad(g, x, need_bias=need_bias, db_out=db_out)
+                        dpw, _ = ops.pw_wgrad(g, x, need_bias=wg_bias, db_out=db_out)
                         grads[l * per] = dpw.reshape(pw_shape)
                     g = ops.dft_inverse(plan, 1, gxh, epi)
                 else:
                     g = fused[0]
                     grads[l * per] = fused[1].reshape(pw_shape)
             elif need_wgrad:
-                dpw, _ = ops.pw_wgrad(g, x, need_bias=need_bias, db_out=db_out)
+                dpw, _ = ops.pw_wgrad(g, x, need_bias=wg_bias, db_out=db_out)
                 grads[l * per] = dpw.reshape(pw_shape)
-        return (g if ctx.needs_input_grad[0] else None, None, None, None,
+        return (g if ctx.needs_input_grad[0] else None, None, None, None, None,
                 dbias.reshape(ctx.bias_shape) if need_bias else None) + tuple(grads)
 
 
-def fno_stack(x, geom: SpecGeom, bias_all, layers, acts):
+def fno_stack(x, geom: SpecGeom, bias_all, layers, acts, norm=None):
     """bias_all: (n_layers, Co, 1, ...) bias of the conv stack; layers: list of (pw_weight, [corners]); acts: activation
-    name (or None) per layer."""
+    name (or None) per layer; norm: None, or (groups, eps, [(weight, bias) per layer]) of the layers' GroupNorm
+    (instance norm: groups = channels; weight = bias = None without affine parameters)."""
     flat = []
-    for pw_w, corners in layers:
+    cfg = None
+    if norm is not None:
+        groups, eps, affine = norm
+        has = {(w is not None, b is not None) for w, b in affine}
+        if len(has) != 1 or len(set(next(iter(has)))) != 1:
+            raise NotImplementedError("fno_stack: every layer's norm needs both affine parameters, or none")
+        cfg = (int(groups), float(eps), affine[0][0] is not None)
+    for l, (pw_w, corners) in enumerate(layers):
         flat += [pw_w] + list(corners)
-    return FNOStackFn.apply(x, geom, tuple(acts), len(layers[0][1]), bias_all, *flat)
+        if cfg is not None and cfg[2]:
+            flat += list(norm[2][l])
+    return FNOStackFn.apply(x, geom, tuple(acts), len(layers[0][1]), cfg, bias_all, *flat)
 
 
 class PointwiseConvFn(torch.autograd.Function):

@@ -169,13 +169,15 @@ class SpectralConv(nn.Module):
     def forward(self, x, indices=0):
         return self.forward_fused(x, indices)
 
-    def forward_fused(self, x, indices=0, pw_weight=None, act=None):
-        """spectral conv + bias [+ 1x1 skip + activation] in one fused pass."""
+    def forward_fused(self, x, indices=0, pw_weight=None, act=None, norm=None):
+        """spectral conv + bias [-> norm] [+ 1x1 skip + activation] in one fused pass; norm: an nn.GroupNorm or
+        InstanceNorm{1,2,3}d module (norm_args)."""
         if x.dim() != 2 + self.order:
             raise ValueError(f"expected a {2 + self.order}-D input (batch, channels, *grid)")
         geom = self._geom(tuple(x.shape[2:]), indices)
         bias = None if self.bias is None else self.bias[indices].reshape(-1)
-        return Fn.spectral_block(x, self.corners(indices), geom, bias=bias, pw_weight=pw_weight, act=act)
+        return Fn.spectral_block(x, self.corners(indices), geom, bias=bias, pw_weight=pw_weight, act=act,
+                                 norm=None if norm is None else _norm_args_or_raise(norm, self.out_channels))
 
     def get_conv(self, indices):
         if self.n_layers == 1:
@@ -259,10 +261,31 @@ class Projection(nn.Module):
                            _act_name(self.non_linearity))
 
 
+def norm_args(m, channels: int):
+    """(groups, eps, weight, bias) of a norm module the spectral path implements, else None: nn.GroupNorm over `channels`
+    channels, or InstanceNorm{1,2,3}d without running statistics (GroupNorm with one channel per group; the statistics are
+    always the instance's own, in training and in eval).  weight / bias are None without affine parameters."""
+    if isinstance(m, nn.GroupNorm):
+        if m.num_channels != channels or channels % m.num_groups != 0:
+            return None
+        return m.num_groups, m.eps, m.weight, m.bias
+    if isinstance(m, nn.modules.instancenorm._InstanceNorm) and not m.track_running_stats and m.num_features == channels:
+        return channels, m.eps, m.weight, m.bias
+    return None
+
+
+def _norm_args_or_raise(m, channels):
+    a = norm_args(m, channels)
+    if a is None:
+        raise NotImplementedError(f"{m} has no native kernel: GroupNorm, or InstanceNorm without running statistics")
+    return a
+
+
 class FNOBlocks(nn.Module):
     """fno_block.py:10-191 restricted to what FNO1d/2d/3d can reach (quirk Q2): linear skips, no MLP, no
-    norm, no preactivation.  Per layer ONE fused pass: spectral conv + bias + 1x1 skip + (GELU iff
-    index < n_layers - index, fno_block.py:149)."""
+    preactivation.  Per layer ONE fused pass: spectral conv + bias [-> instance / group norm] + 1x1 skip + (GELU iff
+    index < n_layers - index, fno_block.py:149).  The norm is applied to the conv's kept-mode spectrum before the
+    inverse transform (ops.spec_norm_fwd), so it adds no pass over the activation."""
 
     def __init__(self, in_channels, out_channels, n_modes, output_scaling_factor=None, n_layers=1,
                  incremental_n_modes=None, use_mlp=False, mlp_dropout=0, mlp_expansion=0.5,
@@ -273,9 +296,13 @@ class FNOBlocks(nn.Module):
         super().__init__()
         if isinstance(n_modes, int):
             n_modes = [n_modes]
-        if use_mlp or norm is not None or preactivation:
-            raise NotImplementedError("native FNOBlocks: use_mlp / norm / preactivation are outside the hot path "
+        if use_mlp or preactivation:
+            raise NotImplementedError("native FNOBlocks: use_mlp / preactivation are outside the hot path "
                                       "(no BASELINE config enables them)")
+        if norm not in (None, "instance_norm", "group_norm"):
+            if norm == "ada_in":
+                raise NotImplementedError("native FNOBlocks: norm='ada_in' is outside the hot path")
+            raise ValueError(f"Got norm={norm} but expected None or one of [instance_norm, group_norm, ada_in]")
         if fno_skip != "linear":
             raise NotImplementedError("native FNOBlocks implements the 'linear' skip (the only one FNO2d reaches)")
         if output_scaling_factor is not None:
@@ -298,13 +325,22 @@ class FNOBlocks(nn.Module):
         Conv = getattr(nn, f"Conv{self.n_dim}d")
         self.fno_skips = nn.ModuleList([Conv(in_channels, out_channels, kernel_size=1, bias=False)
                                         for _ in range(n_layers)])
+        if norm == "instance_norm":     # fno_block.py:94-105 with n_norms = 1 (no MLP), registered after the skips
+            self.norm = nn.ModuleList([getattr(nn, f"InstanceNorm{self.n_dim}d")(num_features=out_channels)
+                                       for _ in range(n_layers)])
+        elif norm == "group_norm":
+            self.norm = nn.ModuleList([nn.GroupNorm(num_groups=1, num_channels=out_channels) for _ in range(n_layers)])
 
     def forward(self, x, index=0):
         act = _act_name(self.non_linearity) if index < (self.n_layers - index) else None
+        norm = None if self.norm is None else self.norm[index]
         if hasattr(self.convs, "forward_fused"):
-            return self.convs.forward_fused(x, index, pw_weight=self.fno_skips[index].weight, act=act)
+            return self.convs.forward_fused(x, index, pw_weight=self.fno_skips[index].weight, act=act, norm=norm)
         # a user-supplied SpectralConv class: keep the reference's composition
-        y = self.convs(x, index) + Fn.pointwise_conv(x, self.fno_skips[index].weight, None, None)
+        y = self.convs(x, index)
+        if norm is not None:
+            y = norm(y)
+        y = y + Fn.pointwise_conv(x, self.fno_skips[index].weight, None, None)
         return self.non_linearity(y) if act is not None else y
 
     @property
@@ -377,14 +413,21 @@ class FNO(nn.Module):
     def forward(self, x):
         x = self.lifting(x)
         blocks = self.fno_blocks
+        norm_args_l = None
+        if isinstance(blocks, FNOBlocks) and blocks.norm is not None and hasattr(blocks.convs, "forward_fused"):
+            norm_args_l = [_norm_args_or_raise(blocks.norm[i], blocks.out_channels) for i in range(self.n_layers)]
         if (isinstance(blocks, FNOBlocks) and hasattr(blocks.convs, "forward_fused") and blocks.convs.bias is not None
-                and blocks.convs.output_scaling_factor is None and x.dim() == 2 + blocks.convs.order):
+                and blocks.convs.output_scaling_factor is None and x.dim() == 2 + blocks.convs.order
+                and (norm_args_l is None or len({(a[0], a[1], a[2] is None) for a in norm_args_l}) == 1)):
             # the whole stack as one autograd node: the backward chains act'(z) into the dx epilogues
             convs = blocks.convs
             geom = convs._geom(tuple(x.shape[2:]), 0)
             acts = [(_act_name(blocks.non_linearity) if i < (blocks.n_layers - i) else None) for i in range(self.n_layers)]
             layers = [(blocks.fno_skips[i].weight, convs.corners(i)) for i in range(self.n_layers)]
-            x = Fn.fno_stack(x, geom, convs.bias, layers, acts)
+            norm = None
+            if norm_args_l is not None:    # one (groups, eps) for the stack, each layer's own weight / bias
+                norm = (norm_args_l[0][0], norm_args_l[0][1], [a[2:] for a in norm_args_l])
+            x = Fn.fno_stack(x, geom, convs.bias, layers, acts, norm=norm)
         else:
             for layer_idx in range(self.n_layers):
                 x = self.fno_blocks(x, layer_idx)

@@ -319,6 +319,44 @@ def mix_dw(plan: Plan, xh: torch.Tensor, gyh: torch.Tensor, like: Sequence[torch
     return grads
 
 
+def spec_norm_fwd(plan: Plan, spec: torch.Tensor, bias: Optional[torch.Tensor], gamma: Optional[torch.Tensor],
+                  beta: Optional[torch.Tensor], groups: int, eps: float):
+    """GroupNorm(groups) of the spectral conv output s = IDFT(spec) + bias, applied to the spectrum (b2no_spec_norm_fwd):
+    returns (the normalised spectrum, for dft_inverse without a bias; the statistics the backward reads)."""
+    _require_cuda(spec, bias, gamma, beta)
+    assert spec.dtype == torch.complex64 and spec.is_contiguous()
+    B, Cc = plan.spec_bc(spec)
+    for t in (bias, gamma, beta):
+        assert t is None or (t.dtype == torch.float32 and t.is_contiguous() and t.numel() == Cc)
+    out = torch.empty_like(spec)
+    stats = torch.empty(2 * B * (Cc + groups), dtype=torch.float32, device=spec.device)
+    check(_lib.lib().b2no_spec_norm_fwd(plan.handle, _ptr(spec), _ptr(bias), _ptr(gamma), _ptr(beta), float(eps), _ptr(out),
+                                        _ptr(stats), B, Cc, int(groups), _stream()), "spec_norm_fwd")
+    return out, stats
+
+
+def spec_norm_bwd(plan: Plan, spec: torch.Tensor, gspec: torch.Tensor, stats: torch.Tensor, gamma: Optional[torch.Tensor],
+                  groups: int, need_bias: bool, need_affine: bool, db_out: Optional[torch.Tensor] = None):
+    """Backward of spec_norm_fwd (b2no_spec_norm_bwd): gspec = dL/d(normalised spectrum) -> (dL/dspec, dbias | None,
+    dgamma | None, dbeta | None).  db_out: contiguous (channels,) destination for dbias."""
+    _require_cuda(spec, gspec)
+    assert gspec.dtype == torch.complex64 and gspec.is_contiguous() and gspec.shape == spec.shape
+    B, Cc = plan.spec_bc(spec)
+    dev = spec.device
+    L = _lib.lib()
+    gout = torch.empty_like(spec)
+    db = None
+    if need_bias:
+        db = db_out if db_out is not None else torch.empty((Cc,), dtype=torch.float32, device=dev)
+        assert db.is_contiguous() and db.numel() == Cc and db.dtype == torch.float32
+    dg = torch.empty((Cc,), dtype=torch.float32, device=dev) if need_affine else None
+    dbt = torch.empty((Cc,), dtype=torch.float32, device=dev) if need_affine else None
+    scratch = torch.empty(int(L.b2no_spec_norm_bwd_scratch_floats(B, Cc)), dtype=torch.float32, device=dev)
+    check(L.b2no_spec_norm_bwd(plan.handle, _ptr(spec), _ptr(gspec), _ptr(stats), _ptr(gamma), _ptr(gout), _ptr(db), _ptr(dg),
+                               _ptr(dbt), _ptr(scratch), B, Cc, int(groups), _stream()), "spec_norm_bwd")
+    return gout, db, dg, dbt
+
+
 def act_bwd(gy: torch.Tensor, z: torch.Tensor, act) -> torch.Tensor:
     gz = torch.empty_like(gy)
     check(_lib.lib().b2no_act_bwd(_ptr(gy), _ptr(z), _ptr(gz), gy.numel(), ACT[act], _stream()), "act_bwd")
