@@ -233,6 +233,25 @@ int64_t b2no_mlp_head_bwd_multi_scratch_floats(int hidden, int out_channels);
 int b2no_mlp_head_bwd_multi(const float* x, const float* w1, const float* b1, const float* w2, const float* g, float* gx,
                             float* gz, float* dw2, float* partial, int batch, int ci, int hidden, int out_channels,
                             int64_t pixels, int b1_per_sample, int act, const float* dact_z, int dact, void* stream);
+/* Channel MLP of an FNO block with its soft-gating skip (fno_block.py:123-170, mlp.py:10-54, skip_connections.py:5-74), per
+ * pixel, u and x (batch, C, pixels), w1 (H, C), b1 (H), w2 (C, H), b2 (C), g (C); b1 / b2 may be NULL:
+ *   s = gelu(w2 gelu(w1 u + b1) + b2) + g x;   y = act(s), and pre = s when act != 0 and pre is not NULL.
+ * The hidden tensor is never written.  Tensor cores only (csrc/tc_channel_mlp.cu): returns B2NO_E_UNSUPPORTED, having written
+ * nothing, where b2no_channel_mlp_supported is 0 (C or H outside 1..64, pixels % 128 != 0, no tensor-core kernels). */
+int b2no_channel_mlp_supported(int channels, int hidden, int64_t pixels);
+int b2no_channel_mlp_fwd(const float* u, const float* x, const float* w1, const float* b1, const float* w2, const float* b2,
+                         const float* g, float* y, float* pre, int batch, int channels, int hidden, int64_t pixels, int act,
+                         void* stream);
+/* Its backward, the hidden activations recomputed on the tensor cores:
+ *   dy = gy act'(pre) (gy when act == 0);  d2 = dy gelu'(a2);  d1 = (w2^T d2) gelu'(a1);  du = w1^T d1;  dx = g dy (the skip's
+ *   share of the block input's gradient; the caller adds it to the other paths');  dg[c] = sum_{b,p} dy x (fixed order);
+ *   h = gelu(a1), d1 (batch, H, pixels) and d2 (batch, C, pixels) for b2no_pw_wgrad: dW1 = sum d1 u^T, db1 = sum d1,
+ *   dW2 = sum d2 h^T, db2 = sum d2.
+ * scratch: b2no_channel_mlp_scratch_floats(C) floats.  Same B2NO_E_UNSUPPORTED rule as the forward. */
+int64_t b2no_channel_mlp_scratch_floats(int channels);
+int b2no_channel_mlp_bwd(const float* u, const float* x, const float* pre, const float* gy, const float* w1, const float* b1,
+                         const float* w2, const float* b2, const float* g, float* du, float* dx, float* h, float* d1, float* d2,
+                         float* dg, float* scratch, int batch, int channels, int hidden, int64_t pixels, int act, void* stream);
 /* RNO gate (rno.py:259): h_next = (1 - z) * h + z2 * hhat, and its backward */
 int b2no_rno_gate_fwd(const float* z, const float* z2, const float* hhat, const float* h, float* out,
                       int64_t n, void* stream);

@@ -9,7 +9,7 @@ from .functional import (spectral_block, pointwise_conv, pointwise_conv2, mlp_he
 from .modules import (  # noqa: F401
     ComplexDenseWeight, SpectralConv, SpectralConv1d, SpectralConv2d, SpectralConv3d, SubConv,
     FactorizedSpectralConv, FactorizedSpectralConv1d, FactorizedSpectralConv2d, FactorizedSpectralConv3d,
-    Lifting, Projection, FNOBlocks, FNO, FNO1d, FNO2d, FNO3d, FNO2dObserver, LpLoss,
+    Lifting, Projection, MLP, SoftGating, FNOBlocks, FNO, FNO1d, FNO2d, FNO3d, FNO2dObserver, LpLoss,
     RnoSpectralConv2d, FourierLayer2d, RNO_cell, RNO_layer, SpectralConvWithFC, SpectralRegressor, RNO2d,
     RNO2dObserver, PinoSpectralConv3d, MultiplicativeNet, PINObserver2d, PlanePredHead, PINObserverFullField,
     PolicyModel2D, PinoSpectralConv2d, PinoFNO2d,

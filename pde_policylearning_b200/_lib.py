@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # B2NO_LIB: load another build, e.g. the parent commit's, for A/B runs in one call
 LIB_PATH = os.environ.get("B2NO_LIB") or os.path.join(_HERE, "libb2no.so")
 CSRC = os.path.join(_HERE, "csrc")
-SOURCES = ["plan.cu", "spectral.cu", "pointwise.cu", "tc_pointwise.cu", "tc_wgrad.cu", "tc_mlp.cu", "tc_head_bwd.cu", "tc_dft.cu", "tc_mix.cu", "tc_peak.cu", "pino_loss.cu", "optim.cu", "spec_norm.cu"]
+SOURCES = ["plan.cu", "spectral.cu", "pointwise.cu", "tc_pointwise.cu", "tc_wgrad.cu", "tc_mlp.cu", "tc_head_bwd.cu", "tc_dft.cu", "tc_mix.cu", "tc_peak.cu", "pino_loss.cu", "optim.cu", "spec_norm.cu", "tc_channel_mlp.cu"]
 
 MAX_DIM = 3
 NORM = {"backward": 0, "forward": 1, "ortho": 2}
@@ -127,6 +127,11 @@ def lib():
     L.b2no_mlp_head_bwd_multi_scratch_floats.restype = i64
     L.b2no_mlp_head_bwd_multi_scratch_floats.argtypes = [i32, i32]
     L.b2no_mlp_head_bwd_multi.argtypes = [vp] * 9 + [i32, i32, i32, i32, i64, i32, i32, vp, i32, vp]
+    L.b2no_channel_mlp_supported.argtypes = [i32, i32, i64]
+    L.b2no_channel_mlp_fwd.argtypes = [vp] * 9 + [i32, i32, i32, i64, i32, vp]
+    L.b2no_channel_mlp_scratch_floats.restype = i64
+    L.b2no_channel_mlp_scratch_floats.argtypes = [i32]
+    L.b2no_channel_mlp_bwd.argtypes = [vp] * 16 + [i32, i32, i32, i64, i32, vp]
     L.b2no_rno_gate_fwd.argtypes = [vp, vp, vp, vp, vp, i64, vp]
     L.b2no_rno_gate_bwd.argtypes = [vp] * 9 + [i64, vp]
     L.b2no_rno_cell_bwd.argtypes = [vp] * 7 + [i32, i32, i64, vp]
@@ -159,6 +164,7 @@ EXPORTS = [
     "b2no_mlp_head_bwd_fused_scratch_floats", "b2no_mlp_head_bwd_fused_supported", "b2no_mlp_head_bwd_fused",
     "b2no_mlp_head_fwd_multi", "b2no_mlp_head_bwd_multi_supported", "b2no_mlp_head_bwd_multi_scratch_floats",
     "b2no_mlp_head_bwd_multi",
+    "b2no_channel_mlp_supported", "b2no_channel_mlp_fwd", "b2no_channel_mlp_scratch_floats", "b2no_channel_mlp_bwd",
     "b2no_rno_gate_fwd", "b2no_rno_gate_bwd", "b2no_rno_cell_bwd", "b2no_rno_reset_bwd", "b2no_rel_l2_sums", "b2no_rel_l2_bwd",
     "b2no_rel_l2_finish", "b2no_rel_l2_bwd_g", "b2no_adam_step", "b2no_gather_segments",
     "b2no_tc_peak_probe", "b2no_pino_residual_scratch_floats", "b2no_pino_residual_fwd", "b2no_pino_residual_bwd",

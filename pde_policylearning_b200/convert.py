@@ -72,8 +72,14 @@ def _convert_pino_conv2d(ref) -> nn.Module:
 
 
 def _convert_fno_blocks(ref):
-    ok = (ref.mlp is None and not ref.preactivation and ref.fno_skip == "linear"
+    ok = (not ref.preactivation and ref.fno_skip == "linear"
           and ref.output_scaling_factor is None and isinstance(ref.convs, M.SpectralConv))
+    # two-layer GELU MLPs without dropout and soft-gating skips without bias run as Fn.channel_mlp (M.mlp_supported), and
+    # not together with a norm; any other MLP keeps the block in torch
+    mlp, mlp_skips = getattr(ref, "mlp", None), getattr(ref, "mlp_skips", None)
+    if ok and mlp is not None:
+        ok = (ref.norm is None and mlp_skips is not None and len(mlp) >= ref.n_layers and len(mlp_skips) >= ref.n_layers
+              and all(M.mlp_supported(mlp[i], mlp_skips[i], ref.out_channels) for i in range(ref.n_layers)))
     # instance / group norms run on the spectrum (M.norm_args); any other norm keeps the block in torch
     if ok and ref.norm is not None:
         ok = len(ref.norm) >= ref.n_layers and all(M.norm_args(m, ref.out_channels) is not None for m in ref.norm)
@@ -84,9 +90,10 @@ def _convert_fno_blocks(ref):
     for k in ("n_modes", "n_dim", "output_scaling_factor", "_incremental_n_modes", "in_channels", "out_channels",
               "n_layers", "joint_factorization", "non_linearity", "fno_skip", "mlp_skip", "fft_norm"):
         setattr(new, k, getattr(ref, k))
-    new.mlp = None
     new.convs = ref.convs
     new.fno_skips = ref.fno_skips
+    new.mlp = mlp                    # the same MLP and gating modules (and Parameters), or None
+    new.mlp_skips = mlp_skips if mlp is not None else None
     new.norm = ref.norm              # the same norm modules (and Parameters), or None
     new.train(ref.training)
     return new

@@ -509,6 +509,59 @@ def mlp_head(x, w1, b1, w2, b2, act="gelu"):
     return pointwise_conv(h, w2, b2, None)
 
 
+class ChannelMlpFn(torch.autograd.Function):
+    """y = act(gelu(W2 gelu(W1 u + b1) + b2) + g x): the channel MLP of an FNO block and its soft-gating skip of the block input
+    x (fno_block.py:123-170, mlp.py:49).  The forward never writes the hidden tensor; the backward recomputes it on the tensor
+    cores (csrc/tc_channel_mlp.cu), returns du, the skip's share of dx and dg, and writes h, d1 and d2 once for the
+    weight-gradient kernel."""
+
+    @staticmethod
+    def forward(ctx, u, x, w1, b1, w2, b2, g, final_act):
+        ops._require_cuda(u, x)
+        u, x = _contig(u.float()), _contig(x.float())
+        w1m = _contig(w1.detach().reshape(w1.shape[0], -1).float())
+        w2m = _contig(w2.detach().reshape(w2.shape[0], -1).float())
+        b1v, b2v, gv = _vec(b1), _vec(b2), _vec(g)
+        y, pre = ops.channel_mlp_fwd(u, x, w1m, b1v, w2m, b2v, gv, final_act, want_pre=any(ctx.needs_input_grad))
+        ctx.act = final_act
+        ctx.shapes = (tuple(w1.shape), None if b1 is None else tuple(b1.shape), tuple(w2.shape),
+                      None if b2 is None else tuple(b2.shape), tuple(g.shape))
+        ctx.save_for_backward(u, x, pre, w1m, b1v, w2m, b2v, gv)
+        return y
+
+    @staticmethod
+    def backward(ctx, gy):
+        u, x, pre, w1m, b1v, w2m, b2v, gv = ctx.saved_tensors
+        gy = _contig(gy.float())
+        du, dx, h, d1, d2, dg = ops.channel_mlp_bwd(u, x, pre, gy, w1m, b1v, w2m, b2v, gv, ctx.act)
+        need = ctx.needs_input_grad
+        dw1 = db1 = dw2 = db2 = None
+        if need[2] or need[3]:
+            dw1, db1 = ops.pw_wgrad(d1, u, need_bias=need[3] and b1v is not None)
+            dw1 = dw1.reshape(ctx.shapes[0])
+            db1 = None if db1 is None else db1.reshape(ctx.shapes[1])
+        if need[4] or need[5]:
+            dw2, db2 = ops.pw_wgrad(d2, h, need_bias=need[5] and b2v is not None)
+            dw2 = dw2.reshape(ctx.shapes[2])
+            db2 = None if db2 is None else db2.reshape(ctx.shapes[3])
+        return (du if need[0] else None, dx if need[1] else None, dw1 if need[2] else None, db1, dw2 if need[4] else None,
+                db2, dg.reshape(ctx.shapes[4]) if need[6] else None, None)
+
+
+def channel_mlp(u, x, w1, b1, w2, b2, g, final_act=None):
+    """act(gelu(W2 gelu(W1 u + b1) + b2) + g x), g the soft-gating weight (1, C, 1...).  Shapes without the channel-MLP kernels
+    (ops.channel_mlp_supported: pixels % 128 != 0, C > 64, H > 64) compose native pointwise convs: the hidden tensor and the
+    MLP output are written, and the gating is a diagonal 1x1 conv in the last conv's two-operand epilogue."""
+    ops._require_cuda(u, x)
+    C, H = u.shape[1], w1.shape[0]
+    if ops.channel_mlp_supported(u, C, H):
+        return ChannelMlpFn.apply(u, x, w1, b1, w2, b2, g, final_act)
+    h = pointwise_conv(u, w1, b1, "gelu")
+    v = pointwise_conv(h, w2, b2, "gelu")
+    eye = torch.eye(C, dtype=torch.float32, device=u.device)
+    return pointwise_conv2(x, torch.diag(g.reshape(-1)), None, final_act, v, eye)
+
+
 class RelL2Fn(torch.autograd.Function):
     """LpLoss.rel with p=2 (libs/utilities3.py:323-334): sum_b or mean_b of ||x_b - y_b|| / ||y_b||.  Three launches in
     all: per-sample sums, the scalar tail (sqrt, ratio, sum) on the device, and dx = g coef_b (x - y)."""

@@ -281,11 +281,76 @@ def _norm_args_or_raise(m, channels):
     return a
 
 
+class MLP(nn.Module):
+    """mlp.py:10-54: n_layers 1x1 convs, the non-linearity after EVERY layer (quirk Q3: `i < n_layers` always holds).
+    FNOBlocks runs its two-layer MLPs through Fn.channel_mlp; this forward is for standalone use."""
+
+    def __init__(self, in_channels, out_channels=None, hidden_channels=None, n_layers=2, n_dim=2, non_linearity=F.gelu,
+                 dropout=0.0, **kwargs):
+        super().__init__()
+        self.n_layers = n_layers
+        self.in_channels = in_channels
+        self.out_channels = in_channels if out_channels is None else out_channels
+        self.hidden_channels = in_channels if hidden_channels is None else hidden_channels
+        self.non_linearity = non_linearity
+        self.dropout = nn.ModuleList([nn.Dropout(dropout) for _ in range(n_layers)]) if dropout > 0.0 else None
+        Conv = getattr(nn, f"Conv{n_dim}d")
+        self.fcs = nn.ModuleList()
+        for i in range(n_layers):
+            ci = self.in_channels if i == 0 else self.hidden_channels
+            co = self.out_channels if i == n_layers - 1 else self.hidden_channels
+            self.fcs.append(Conv(ci, co, 1))
+
+    def forward(self, x):
+        for i, fc in enumerate(self.fcs):
+            x = Fn.pointwise_conv(x, fc.weight, fc.bias, _act_name(self.non_linearity))
+            if self.dropout is not None:
+                x = self.dropout[i](x)
+        return x
+
+
+class SoftGating(nn.Module):
+    """skip_connections.py:37-74: x * weight (+ bias), weight (1, C, 1...) initialised to ones."""
+
+    def __init__(self, in_features, out_features=None, n_dim=2, bias=False):
+        super().__init__()
+        if out_features is not None and in_features != out_features:
+            raise ValueError(f"Got in_features={in_features} and out_features={out_features} "
+                             "but these two must be the same for soft-gating")
+        self.in_features, self.out_features, self.n_dim = in_features, out_features, n_dim
+        self.weight = nn.Parameter(torch.ones(1, self.in_features, *(1,) * n_dim))
+        self.bias = nn.Parameter(torch.ones(1, self.in_features, *(1,) * n_dim)) if bias else None
+
+    def forward(self, x):
+        # a diagonal 1x1 conv on the native pointwise kernel
+        return Fn.pointwise_conv(x, torch.diag(self.weight.reshape(-1)),
+                                 None if self.bias is None else self.bias.reshape(-1), None)
+
+
+def mlp_supported(mlp, skip, channels: int) -> bool:
+    """True for the channel MLP Fn.channel_mlp implements (fno_block.py:123-170 with use_mlp): two 1x1 convs with biases,
+    C -> H -> C, GELU, no dropout, and a soft-gating skip without bias."""
+    if not (hasattr(mlp, "fcs") and len(mlp.fcs) == 2 and getattr(mlp, "dropout", None) is None
+            and isinstance(skip, nn.Module) and type(skip).__name__ == "SoftGating" and getattr(skip, "bias", None) is None):
+        return False
+    try:
+        if _act_name(mlp.non_linearity) != "gelu":
+            return False
+    except NotImplementedError:
+        return False
+    fc1, fc2 = mlp.fcs
+    return (fc1.weight.shape[1] == channels and fc2.weight.shape[0] == channels and fc2.weight.shape[1] == fc1.weight.shape[0]
+            and fc1.bias is not None and fc2.bias is not None and tuple(skip.weight.shape[:2]) == (1, channels))
+
+
 class FNOBlocks(nn.Module):
-    """fno_block.py:10-191 restricted to what FNO1d/2d/3d can reach (quirk Q2): linear skips, no MLP, no
-    preactivation.  Per layer ONE fused pass: spectral conv + bias [-> instance / group norm] + 1x1 skip + (GELU iff
-    index < n_layers - index, fno_block.py:149).  The norm is applied to the conv's kept-mode spectrum before the
-    inverse transform (ops.spec_norm_fwd), so it adds no pass over the activation."""
+    """fno_block.py:10-191 restricted to what FNO1d/2d/3d can reach (quirk Q2): linear skips, no preactivation.  Per layer
+    ONE fused pass: spectral conv + bias [-> instance / group norm] + 1x1 skip + (GELU iff index < n_layers - index,
+    fno_block.py:149).  The norm is applied to the conv's kept-mode spectrum before the inverse transform
+    (ops.spec_norm_fwd), so it adds no pass over the activation.  With use_mlp (fno_block.py:123-170) the activation is
+    always applied, then the channel MLP C -> round(C mlp_expansion) -> C (GELU after both convs), its soft-gating skip of
+    the block input and the activation for every layer but the last run as one more fused node (Fn.channel_mlp); use_mlp
+    with a norm, MLP dropout and the 'linear' / 'identity' MLP skips raise."""
 
     def __init__(self, in_channels, out_channels, n_modes, output_scaling_factor=None, n_layers=1,
                  incremental_n_modes=None, use_mlp=False, mlp_dropout=0, mlp_expansion=0.5,
@@ -296,9 +361,15 @@ class FNOBlocks(nn.Module):
         super().__init__()
         if isinstance(n_modes, int):
             n_modes = [n_modes]
-        if use_mlp or preactivation:
-            raise NotImplementedError("native FNOBlocks: use_mlp / preactivation are outside the hot path "
-                                      "(no BASELINE config enables them)")
+        if preactivation:
+            raise NotImplementedError("native FNOBlocks: preactivation is outside the hot path (no BASELINE config enables it)")
+        if use_mlp and norm is not None:
+            # the second norm would act on the MLP output, which is not band-limited: no spectral form
+            raise NotImplementedError("native FNOBlocks: use_mlp together with a norm has no native kernel")
+        if use_mlp and mlp_dropout > 0:
+            raise NotImplementedError("native FNOBlocks: mlp_dropout > 0 has no native kernel")
+        if use_mlp and mlp_skip != "soft-gating":
+            raise NotImplementedError("native FNOBlocks: the MLP skip runs natively as 'soft-gating' only")
         if norm not in (None, "instance_norm", "group_norm"):
             if norm == "ada_in":
                 raise NotImplementedError("native FNOBlocks: norm='ada_in' is outside the hot path")
@@ -315,6 +386,7 @@ class FNOBlocks(nn.Module):
         self.non_linearity = non_linearity
         self.fno_skip, self.mlp_skip, self.fft_norm = fno_skip, mlp_skip, fft_norm
         self.mlp = None
+        self.mlp_skips = None
         self.norm = None
         self.convs = SpectralConv(in_channels, out_channels, self.n_modes, output_scaling_factor=None,
                                   incremental_n_modes=incremental_n_modes, rank=rank, fft_norm=fft_norm,
@@ -325,6 +397,10 @@ class FNOBlocks(nn.Module):
         Conv = getattr(nn, f"Conv{self.n_dim}d")
         self.fno_skips = nn.ModuleList([Conv(in_channels, out_channels, kernel_size=1, bias=False)
                                         for _ in range(n_layers)])
+        if use_mlp:     # fno_block.py:75-84, registered after the fno skips
+            self.mlp = nn.ModuleList([MLP(in_channels=out_channels, hidden_channels=int(round(out_channels * mlp_expansion)),
+                                          dropout=mlp_dropout, n_dim=self.n_dim) for _ in range(n_layers)])
+            self.mlp_skips = nn.ModuleList([SoftGating(in_channels, out_channels, n_dim=self.n_dim) for _ in range(n_layers)])
         if norm == "instance_norm":     # fno_block.py:94-105 with n_norms = 1 (no MLP), registered after the skips
             self.norm = nn.ModuleList([getattr(nn, f"InstanceNorm{self.n_dim}d")(num_features=out_channels)
                                        for _ in range(n_layers)])
@@ -332,6 +408,8 @@ class FNOBlocks(nn.Module):
             self.norm = nn.ModuleList([nn.GroupNorm(num_groups=1, num_channels=out_channels) for _ in range(n_layers)])
 
     def forward(self, x, index=0):
+        if self.mlp is not None:
+            return self._forward_mlp(x, index)
         act = _act_name(self.non_linearity) if index < (self.n_layers - index) else None
         norm = None if self.norm is None else self.norm[index]
         if hasattr(self.convs, "forward_fused"):
@@ -342,6 +420,18 @@ class FNOBlocks(nn.Module):
             y = norm(y)
         y = y + Fn.pointwise_conv(x, self.fno_skips[index].weight, None, None)
         return self.non_linearity(y) if act is not None else y
+
+    def _forward_mlp(self, x, index):
+        """fno_block.py:123-170 with an MLP: u = act(conv(x) + skip x) (the activation always on), then
+        y = gelu(fc2 gelu(fc1 u)) + g x, followed by act for every layer but the last."""
+        act = _act_name(self.non_linearity)
+        if hasattr(self.convs, "forward_fused"):
+            u = self.convs.forward_fused(x, index, pw_weight=self.fno_skips[index].weight, act=act)
+        else:
+            u = self.non_linearity(self.convs(x, index) + Fn.pointwise_conv(x, self.fno_skips[index].weight, None, None))
+        fc1, fc2 = self.mlp[index].fcs
+        return Fn.channel_mlp(u, x, fc1.weight, fc1.bias, fc2.weight, fc2.bias, self.mlp_skips[index].weight,
+                              act if index < self.n_layers - 1 else None)
 
     @property
     def incremental_n_modes(self):
@@ -385,6 +475,11 @@ class FNO(nn.Module):
         super().__init__()
         if domain_padding is not None and domain_padding > 0:
             raise NotImplementedError("native FNO: domain_padding is outside the hot path (no config enables it)")
+        if use_mlp:
+            # the mirrored model classes keep rejecting use_mlp; channel-MLP blocks run natively as FNOBlocks(use_mlp=True):
+            # the blocks of a converted reference model (convert_), or blocks assigned to fno_blocks, run by forward() below
+            raise NotImplementedError("native FNO: use_mlp is not built by FNO / FNO1d / FNO2d / FNO3d; build the model with "
+                                      "the reference classes and convert_() it, or assign FNOBlocks(use_mlp=True) to fno_blocks")
         self.n_dim = len(n_modes)
         self.n_modes = n_modes
         self.hidden_channels = hidden_channels
@@ -416,7 +511,8 @@ class FNO(nn.Module):
         norm_args_l = None
         if isinstance(blocks, FNOBlocks) and blocks.norm is not None and hasattr(blocks.convs, "forward_fused"):
             norm_args_l = [_norm_args_or_raise(blocks.norm[i], blocks.out_channels) for i in range(self.n_layers)]
-        if (isinstance(blocks, FNOBlocks) and hasattr(blocks.convs, "forward_fused") and blocks.convs.bias is not None
+        if (isinstance(blocks, FNOBlocks) and blocks.mlp is None and hasattr(blocks.convs, "forward_fused")
+                and blocks.convs.bias is not None
                 and blocks.convs.output_scaling_factor is None and x.dim() == 2 + blocks.convs.order
                 and (norm_args_l is None or len({(a[0], a[1], a[2] is None) for a in norm_args_l}) == 1)):
             # the whole stack as one autograd node: the backward chains act'(z) into the dx epilogues

@@ -514,6 +514,40 @@ def mlp_head_bwd_multi(x, w1, b1, w2, g, act="gelu", want_gz=True, dact_z=None, 
     return gx, gz, dw2
 
 
+def channel_mlp_supported(x: torch.Tensor, channels: int, hidden: int) -> bool:
+    """True when the channel-MLP kernels (b2no_channel_mlp_fwd / _bwd) run for x: a CUDA tensor and a supported shape."""
+    return x.is_cuda and bool(_lib.lib().b2no_channel_mlp_supported(channels, hidden, math.prod(x.shape[2:])))
+
+
+def channel_mlp_fwd(u, x, w1, b1, w2, b2, g, act=None, want_pre=False):
+    """s = gelu(W2 gelu(W1 u + b1) + b2) + g x, y = act(s) (b2no_channel_mlp_fwd): returns (y, pre | None), pre = s written when
+    want_pre and act is set.  Every tensor contiguous float32; w1 (H, C), w2 (C, H), g (C)."""
+    B, Cc = u.shape[:2]
+    hidden = w1.shape[0]
+    y = torch.empty_like(u)
+    pre = torch.empty_like(u) if (want_pre and ACT[act]) else None
+    check(_lib.lib().b2no_channel_mlp_fwd(_ptr(u), _ptr(x), _ptr(w1), _ptr(b1), _ptr(w2), _ptr(b2), _ptr(g), _ptr(y), _ptr(pre),
+                                          B, Cc, hidden, math.prod(u.shape[2:]), ACT[act], _stream()), "channel_mlp_fwd")
+    return y, pre
+
+
+def channel_mlp_bwd(u, x, pre, gy, w1, b1, w2, b2, g, act=None):
+    """Backward of channel_mlp_fwd (b2no_channel_mlp_bwd): returns (du, dx (the skip's share), h, d1, d2, dg)."""
+    B, Cc = u.shape[:2]
+    grid = tuple(u.shape[2:])
+    hidden = w1.shape[0]
+    L = _lib.lib()
+    du, dx, d2 = torch.empty_like(u), torch.empty_like(u), torch.empty_like(u)
+    h = torch.empty((B, hidden) + grid, dtype=torch.float32, device=u.device)
+    d1 = torch.empty_like(h)
+    dg = torch.empty((Cc,), dtype=torch.float32, device=u.device)
+    scratch = torch.empty(int(L.b2no_channel_mlp_scratch_floats(Cc)), dtype=torch.float32, device=u.device)
+    check(L.b2no_channel_mlp_bwd(_ptr(u), _ptr(x), _ptr(pre), _ptr(gy), _ptr(w1), _ptr(b1), _ptr(w2), _ptr(b2), _ptr(g), _ptr(du),
+                                 _ptr(dx), _ptr(h), _ptr(d1), _ptr(d2), _ptr(dg), _ptr(scratch), B, Cc, hidden, math.prod(grid),
+                                 ACT[act], _stream()), "channel_mlp_bwd")
+    return du, dx, h, d1, d2, dg
+
+
 def rno_gate_fwd(z, z2, hh, h):
     out = torch.empty_like(h)
     check(_lib.lib().b2no_rno_gate_fwd(_ptr(z), _ptr(z2), _ptr(hh), _ptr(h), _ptr(out), h.numel(), _stream()), "gate")
